@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the orgscorer hot path (contract: see the task statement / DESIGN.md section 6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the whole hot path (K1..K10) over one batch of synthetic contigs of
 BASELINE.json's configs[1] shape (cfg2: 100k contigs per GPU, 2-8 genes, ~50 hits/gene, 5k species).
@@ -17,6 +17,9 @@ N > 1    : one process per GPU (torchrun).  ONE global batch (N tiles of the 100
 `strong` : configs[2] (1M contigs total, 8-level taxonomy) cut over the N ranks the same way (strong scaling).
 --impl reference : the UNMODIFIED reference (oracle/_ref, installed by oracle/build_ref.py) on all host cores, one
            process per core, on a bounded sample of the same workload; the numpy port if the install is missing.
+--dump-outputs DIR : after the timed steps, the results of the last device-resident step (what `value` timed; rank 0's
+           shard when N > 1) as DIR/<name>.npy in float64, at most 64 MB in all.  The workload is seeded, so two builds
+           can be compared array for array.
 """
 
 import argparse
@@ -57,7 +60,47 @@ def parse_args():
     ap.add_argument("--exact", action="store_true", help="exact pipeline for every contig (bit-exact crit / rank)")
     ap.add_argument("--wide", action="store_true", help="e2e leg with the wide 29 B/hit wire format")
     ap.add_argument("--opt", action="append", default=[], help="engine option name=value (wfl_set_option)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's result arrays to DIR/<name>.npy (float64, <= 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA engine's results: it needs --impl ours")
+    return args
+
+
+DUMP_BYTES = 64 * 10 ** 6   # --dump-outputs: all .npy files together, headers included
+NPY_HEADER = 128            # bytes np.save writes before the data of a 1-d or 2-d array
+
+
+def dump_outputs(res, out_dir, limit=DUMP_BYTES):
+    """Every non-empty result array as <out_dir>/<name>.npy in float64 (exact for the engine's integer outputs); an array
+    without elements (ann_winner of a workload without annotation systems) carries no output and is not written.  When the
+    whole would exceed `limit`, each array larger than a common byte budget keeps that many rows, chosen by a generator
+    seeded with 0; arrays of the same length (the per-contig ones, the per-locus ones) therefore keep the same rows, and
+    small arrays such as call_counts stay whole.  Returns the bytes written."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v) for k, v in res.items() if np.asarray(v).size > 0}
+    room = limit - NPY_HEADER * len(arrays)
+    sizes = sorted(8 * a.size for a in arrays.values())
+    cap = room
+    if sum(sizes) > room:   # largest per-array budget `cap` with sum(min(size, cap)) <= room
+        left, n_big = room, len(sizes)
+        for s in sizes:
+            if s * n_big > left:
+                break
+            left, n_big = left - s, n_big - 1
+        cap = left // n_big
+    written = 0
+    for name, a in arrays.items():
+        if 8 * a.size > cap:
+            keep = cap // (8 * (a.size // len(a)))
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, a.astype(np.float64))
+        written += os.path.getsize(path)
+    return written
 
 
 # --------------------------------------------------------------------------------------------
@@ -547,6 +590,9 @@ def main():
                                                 "guard_trips", "refined_groups", "host_syncs")},
         }
         print(json.dumps(line))
+    if args.dump_outputs and rank == 0:   # `res`: plain host arrays of the last resident step, untouched by the later legs
+        nbytes = dump_outputs(res, args.dump_outputs)
+        print("dumped {:.1f} MB of results to {}".format(nbytes / 1e6, args.dump_outputs), file=sys.stderr)
     eng.close()
     if dist is not None:
         dist.destroy_process_group()
@@ -578,7 +624,7 @@ def strong_leg(args, eng, dist, world, rank, barrier, rtol):
     eng.set_params(params3)
     eng.set_taxonomy(tax3)
     e2e = E2E(eng, shard3, params3, tax3, dist, args.wide)
-    steps = max(2, min(args.steps, 4))
+    steps = args.steps
     ms = timed_e2e(e2e, steps, 1, barrier)
     st = eng.stats()
     parity = None
