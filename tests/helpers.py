@@ -37,6 +37,24 @@ def compare_results(ref, got, score_rtol=0.0):
     return diffs
 
 
+def near_print_edge(x, tol=1e-11):
+    """True if x lies within `tol` of a value that prints differently on either side at 4 decimals (x.xxxx5)."""
+    y = float(x) * 1e4
+    return abs(y - np.floor(y) - 0.5) <= tol * 1e4
+
+
+def compare_printed(ref, got):
+    """crit / rank of every contig the reference classifies, as the TSV writer prints them (4 decimals)."""
+    from waafle_b200.utils import format_field
+    diffs = []
+    for c in np.nonzero(np.asarray(ref["call"]) != 0)[0]:
+        for k in ("crit", "rank"):
+            a, b = format_field(float(ref[k][c])), format_field(float(got[k][c]))
+            if a != b:
+                diffs.append((k, int(c), a, b, float(ref[k][c]).hex(), float(got[k][c]).hex()))
+    return diffs
+
+
 def load_json(name):
     path = os.path.join(GOLDEN, name)
     if path.endswith(".gz"):

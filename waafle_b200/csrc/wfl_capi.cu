@@ -1000,7 +1000,18 @@ __global__ void wfl_pack_results_kernel(const PackArgs a) {
     const int64_t n16 = (a.bytes[sec] + 15) / 16;
     const uint4 *s = static_cast<const uint4 *>(a.src[sec]);
     uint4 *d = reinterpret_cast<uint4 *>(a.dst + a.off[sec]);
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += (int64_t)gridDim.x * blockDim.x) d[i] = s[i];
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t rem = a.bytes[sec] - 16 * i;
+        if (rem >= 16) {
+            d[i] = s[i];
+        } else {   // a section's last, partial chunk: the padding is zero (and nothing past the section is read)
+            uint4 v = make_uint4(0u, 0u, 0u, 0u);
+            const unsigned char *sb = reinterpret_cast<const unsigned char *>(s + i);
+            unsigned char *vb = reinterpret_cast<unsigned char *>(&v);
+            for (int k = 0; k < (int)rem; ++k) vb[k] = sb[k];
+            d[i] = v;
+        }
+    }
     if (sec == 0 && blockIdx.x == 0 && threadIdx.x < 8) reinterpret_cast<int64_t *>(a.dst)[threadIdx.x] = a.header[threadIdx.x];
 }
 
