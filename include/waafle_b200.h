@@ -37,7 +37,8 @@ typedef enum {
     WFL_ERR_CUDA = -2,      /* CUDA runtime error (text in wfl_last_error)   */
     WFL_ERR_STATE = -3,     /* params / taxonomy / batch not set             */
     WFL_ERR_CAPACITY = -4,  /* caller-provided output buffer too small       */
-    WFL_ERR_RUNAWAY = -5    /* >100 taxonomy lifts (reference: wu.die, waafle_orgscorer.py:580-581) */
+    WFL_ERR_RUNAWAY = -5,   /* >100 taxonomy lifts (reference: wu.die, waafle_orgscorer.py:580-581) */
+    WFL_ERR_RANGE = -6      /* a score outside the range the details formatter prints exactly (|x| < 2^53)  */
 } wfl_status;
 
 /* Engine-relevant CLI flags (waafle_orgscorer.py:188-296, waafle_genecaller.py:83-101;
@@ -266,6 +267,24 @@ int  wfl_parser_genes_fetch(wfl_parser *p, int64_t *gene_off, int32_t *start, in
  * produced. */
 int64_t wfl_download_details(wfl_engine *e, int32_t *contig, int32_t *iteration, int32_t *clade, int32_t *locus, double *score,
                              int64_t capacity);
+/* The details table as text, built on the device from the dump of the last run:
+ *     contig \t iteration \t clade \t gene_scores \t gene_spans \n
+ * per contig (in the caller's order), evaluated level (iteration = max(1, evaluation index)) and clade (ascending node
+ * index), scores printed like Python's "{:.3f}", spans as write_details (:773-791) derives them from the site arrays.
+ * wfl_set_clade_names: the names of the taxonomy's nodes, name i = blob[off[i], off[i+1]); once per wfl_set_taxonomy.
+ * wfl_details_prepare: `order` lists n_order distinct contig indices of the batch (contigs not listed, and contigs that
+ * were never evaluated, have no rows); contig c is named names[names_off[c], names_off[c+1]).  Returns the table's size
+ * in bytes; bytes_before[r] (n_order + 1 entries, NULL = skip) = bytes of the rows of order[0, r).  Errors: WFL_ERR_STATE
+ * without a details run or without clade names, WFL_ERR_CAPACITY when the dump overflowed its capacity, WFL_ERR_RANGE
+ * when a score cannot be printed exactly.
+ * wfl_details_text: the rows of order[r0, r1); returns their size and writes them to `buf` when capacity >= size (so a
+ * large table is fetched in bounded pieces).  WFL_ERR_STATE without a prepare since the last run.
+ * ms_* (NULL = skip): CUDA-event times of the text kernels and of the copy to `buf`. */
+int  wfl_set_clade_names(wfl_engine *e, int32_t n_nodes, const char *blob, const int64_t *off);
+int64_t wfl_details_prepare(wfl_engine *e, int64_t n_order, const int32_t *order, const char *names, const int64_t *names_off,
+                            int64_t *bytes_before, float *ms_kernels);
+int64_t wfl_details_text(wfl_engine *e, int64_t r0, int64_t r1, char *buf, int64_t capacity, float *ms_kernels,
+                         float *ms_d2h);
 
 /* ---- waafle_genecaller on the device (SURVEY 8f): gene calls from BLAST hits ------------------------------------
  * Replaces the per-contig body of waafle/waafle_genecaller.py:207-230 (hits2ints :107-113, overlap_intervals :137-168,
@@ -287,6 +306,9 @@ void wfl_host_free(void *p);
  * (clade, retained-locus index, score); returns the number of triples or <0. */
 int64_t wfl_debug_gene_scores(wfl_engine *e, int64_t contig, int32_t *clade, int32_t *locus,
                               double *score, int64_t capacity);
+/* Test hook: x[i] printed by the details table's "{:.3f}" formatter into text[24 i, 24 i + len[i]); returns n, or
+ * WFL_ERR_RANGE if some x[i] lies outside |x| < 2^53 (len[i] = -1 there). */
+int64_t wfl_debug_format_scores(wfl_engine *e, const double *x, int64_t n, char *text, int32_t *len);
 
 #ifdef __cplusplus
 }

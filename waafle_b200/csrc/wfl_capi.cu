@@ -54,6 +54,11 @@ struct wfl_engine {
     Buf fb_list, fast_scratch, fast_wq, blob, status_tmp;
     Buf det[6];                          // --write-details dump: contig, iteration, clade, locus, score, count
     int64_t det_cap = 0, det_used = 0;
+    // --write-details text (wfl_details.cu): clade names of the taxonomy, state of the last wfl_details_prepare
+    Buf tname, tname_off, cname, cname_off, dt_found, dt_seg, dt_off, dt_bytes, dt_scratch, dt_defer[2], dt_ctr, dt_text;
+    bool have_tnames = false, dt_ready = false;
+    std::vector<int64_t> dt_seg_off;     // [segments + 1] byte offset of every segment in the table
+    std::vector<int64_t> dt_rank_seg;    // [n_order + 1] first segment of every position of the caller's contig order
     size_t fast_scratch_slot = 0;        // bytes of fast-kernel scratch per compute stream
     bool chunks_pool_bound = false;      // the current chunk plan was cut for the exact pipeline's workspace pool
     int plan_nmax = 0;
@@ -847,6 +852,7 @@ int run_kernels(wfl_engine *e, bool streamed, wfl_results *out) {
         return WFL_ERR_STATE;
     }
     const float h2d = e->stats.ms_h2d;
+    e->dt_ready = false;
     e->stats = wfl_stats{};
     e->stats.ms_h2d = h2d;
     e->stats.contigs = e->n;
@@ -1026,6 +1032,74 @@ int64_t results_layout(int64_t n, int64_t nl, int32_t S, int64_t members, int64_
     return o;
 }
 
+// ---- --write-details text (wfl_details.cu) ----
+DetTextArgs details_args(wfl_engine *e) {
+    DetTextArgs a{};
+    a.b = e->b; a.t = e->tax; a.P = e->P;
+    a.anc = static_cast<const int *>(e->anc.p);
+    a.anc_rows = e->anc_rows;
+    a.dc = static_cast<const int32_t *>(e->det[0].p);
+    a.di = static_cast<const int32_t *>(e->det[1].p);
+    a.dc_clade = static_cast<const int32_t *>(e->det[2].p);
+    a.dl = static_cast<const int32_t *>(e->det[3].p);
+    a.ds = static_cast<const double *>(e->det[4].p);
+    a.seg = static_cast<const DetSeg *>(e->dt_seg.p);
+    a.cname = static_cast<const char *>(e->cname.p);
+    a.cname_off = static_cast<const int64_t *>(e->cname_off.p);
+    a.tname = static_cast<const char *>(e->tname.p);
+    a.tname_off = static_cast<const int64_t *>(e->tname_off.p);
+    a.seg_bytes = static_cast<long long *>(e->dt_bytes.p);
+    a.text_off = static_cast<const long long *>(e->dt_off.p);
+    unsigned long long *ctr = static_cast<unsigned long long *>(e->dt_ctr.p);
+    a.max_need = ctr;
+    a.n_defer = reinterpret_cast<unsigned int *>(ctr + 1);
+    a.err = reinterpret_cast<unsigned int *>(ctr + 2);
+    a.n_found = reinterpret_cast<unsigned int *>(ctr + 3);
+    return a;
+}
+
+// The rows kernel over the segments [s0, s1): every warp of the first launch owns a 32 KB scratch slice; segments
+// that need more (many hits or groups) go to a second launch whose slices fit the largest of them.  `text` null: the
+// length pass (bytes of every segment); otherwise the segments' text at text_off - text_off[s0].
+int details_rows(wfl_engine *e, int64_t s0, int64_t s1, char *text) {
+    if (s1 <= s0) return WFL_OK;
+    int rc;
+    const long long slice1 = 32 << 10, warps1 = (long long)e->sm_count * 64;
+    const size_t n = (size_t)(s1 - s0);
+    int *defer;
+    char *scratch;
+    if ((rc = outbuf(e, e->dt_defer[0], n, &defer)) || (rc = outbuf(e, e->dt_defer[1], n, &defer)) ||
+        (rc = outbuf(e, e->dt_scratch, (size_t)(slice1 * warps1), &scratch)))
+        return rc;
+    DetTextArgs a = details_args(e);
+    a.text = text;
+    a.text_base = e->dt_seg_off[(size_t)s0];
+    CU(cudaMemsetAsync(e->dt_ctr.p, 0, 2 * sizeof(unsigned long long), e->stream));
+    a.s0 = s0; a.n_list = (long long)n; a.list = nullptr;
+    a.scratch = scratch; a.slice = slice1;
+    a.defer = static_cast<int *>(e->dt_defer[0].p);
+    launch_details_rows(a, std::min<long long>(warps1, ((long long)n + 7) & ~7ll), e->stream);
+    CU(cudaGetLastError());
+    e->stats.kernel_launches++;
+    unsigned long long hc[2] = {0, 0};
+    CU(cudaMemcpyAsync(hc, e->dt_ctr.p, sizeof hc, cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    const long long n_defer = (long long)(hc[1] & 0xffffffffull);
+    if (n_defer == 0) return WFL_OK;
+    const long long slice2 = ((long long)hc[0] + 255) & ~255ll;
+    // whole blocks of 8 warps: every launched warp owns a slice
+    const long long warps2 = (std::max<long long>(1, std::min<long long>(n_defer, (1ll << 30) / slice2)) + 7) & ~7ll;
+    if ((rc = outbuf(e, e->dt_scratch, (size_t)(slice2 * warps2), &scratch))) return rc;
+    a.list = static_cast<const int *>(e->dt_defer[0].p);
+    a.n_list = n_defer;
+    a.scratch = scratch; a.slice = slice2;
+    a.defer = static_cast<int *>(e->dt_defer[1].p);
+    launch_details_rows(a, warps2, e->stream);
+    CU(cudaGetLastError());
+    e->stats.kernel_launches++;
+    return WFL_OK;
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------
@@ -1111,6 +1185,9 @@ void wfl_destroy(wfl_engine *e) {
     for (auto &b : e->dbg) fr(b);
     fr(e->anc); fr(e->ctr); fr(e->work); fr(e->scratch); fr(e->plan_index); fr(e->plan_data);
     for (auto &b : e->det) fr(b);
+    for (Buf *b : {&e->tname, &e->tname_off, &e->cname, &e->cname_off, &e->dt_found, &e->dt_seg, &e->dt_off, &e->dt_bytes,
+                   &e->dt_scratch, &e->dt_defer[0], &e->dt_defer[1], &e->dt_ctr, &e->dt_text})
+        fr(*b);
     fr(e->fb_list); fr(e->fast_scratch); fr(e->fast_wq); fr(e->blob); fr(e->status_tmp);
     for (int q = 0; q < 2; ++q) { fr(e->pipe_pool[q]); fr(e->pipe_lists[q]); fr(e->pipe_cnt[q]); fr(e->pipe_wq[q]); }
     fr(e->pipe_ctg);
@@ -1199,6 +1276,7 @@ int wfl_set_taxonomy(wfl_engine *e, int32_t n_nodes, const int32_t *parent, cons
     e->tax.root = root_idx;
     e->tax.unknown = unknown_idx;
     e->have_tax = true;
+    e->have_tnames = e->dt_ready = false;
     e->have_batch = e->have_results = false;
     return WFL_OK;
 }
@@ -1339,6 +1417,168 @@ int64_t wfl_debug_gene_scores(wfl_engine *e, int64_t contig, int32_t *clade, int
     }
     e->have_results = false;
     return cnt;
+}
+
+int wfl_set_clade_names(wfl_engine *e, int32_t n_nodes, const char *blob, const int64_t *off) {
+    if (!e) return WFL_ERR_ARG;
+    if (!e->have_tax || n_nodes != e->tax.n_nodes) { set_err(e, "clade names need the taxonomy they name"); return WFL_ERR_STATE; }
+    if (!off || off[0] != 0 || (off[n_nodes] > 0 && !blob)) { set_err(e, "bad clade name blob"); return WFL_ERR_ARG; }
+    for (int32_t i = 0; i < n_nodes; ++i)
+        if (off[i + 1] < off[i]) { set_err(e, "clade name offsets are not monotone"); return WFL_ERR_ARG; }
+    CU(cudaSetDevice(e->device));
+    int rc;
+    const char *d1;
+    const int64_t *d2;
+    if ((rc = upload(e, e->tname, blob, (size_t)off[n_nodes], &d1)) || (rc = upload(e, e->tname_off, off, (size_t)n_nodes + 1, &d2)))
+        return rc;
+    CU(cudaStreamSynchronize(e->stream));
+    e->have_tnames = true;
+    return WFL_OK;
+}
+
+int64_t wfl_details_prepare(wfl_engine *e, int64_t n_order, const int32_t *order, const char *names, const int64_t *names_off,
+                            int64_t *bytes_before, float *ms_kernels) {
+    if (!e) return WFL_ERR_ARG;
+    e->dt_ready = false;
+    if (!e->have_results || e->det_cap <= 0 || !e->det[5].p) { set_err(e, "no details: set option details=<capacity> and run"); return WFL_ERR_STATE; }
+    if (!e->have_tnames) { set_err(e, "no clade names: wfl_set_clade_names after wfl_set_taxonomy"); return WFL_ERR_STATE; }
+    if (n_order < 0 || (n_order && !order) || !names_off || names_off[0] != 0 || (names_off[e->n] > 0 && !names)) {
+        set_err(e, "bad contig order or names");
+        return WFL_ERR_ARG;
+    }
+    std::vector<int64_t> rank((size_t)e->n, -1);
+    for (int64_t r = 0; r < n_order; ++r) {
+        if (order[r] < 0 || order[r] >= e->n || rank[(size_t)order[r]] >= 0) {
+            set_err(e, "contig order: index out of range or repeated at position %lld", (long long)r);
+            return WFL_ERR_ARG;
+        }
+        rank[(size_t)order[r]] = r;
+    }
+    for (int64_t c = 0; c < e->n; ++c)
+        if (names_off[c + 1] < names_off[c]) { set_err(e, "contig name offsets are not monotone"); return WFL_ERR_ARG; }
+    CU(cudaSetDevice(e->device));
+    unsigned long long cnt = 0;
+    CU(cudaMemcpy(&cnt, e->det[5].p, sizeof cnt, cudaMemcpyDeviceToHost));
+    if ((long long)cnt > e->det_cap) { set_err(e, "details dump overflowed: run again with details >= %llu", cnt); return WFL_ERR_CAPACITY; }
+    int rc;
+    const char *d1;
+    const int64_t *d2;
+    unsigned long long *ctr;
+    DetSeg *found;
+    if ((rc = upload(e, e->cname, names, (size_t)names_off[e->n], &d1)) ||
+        (rc = upload(e, e->cname_off, names_off, (size_t)e->n + 1, &d2)) || (rc = outbuf(e, e->dt_ctr, 4, &ctr)) ||
+        (rc = outbuf(e, e->dt_found, (size_t)cnt, &found)))
+        return rc;
+    CU(cudaEventRecord(e->ev[0], e->stream));
+    CU(cudaMemsetAsync(ctr, 0, 4 * sizeof(unsigned long long), e->stream));
+    DetTextArgs a = details_args(e);
+    a.n_dump = (long long)cnt;
+    a.found = found;
+    launch_details_segments(a, e->stream);
+    CU(cudaGetLastError());
+    e->stats.kernel_launches++;
+    unsigned long long hc[4];
+    CU(cudaMemcpyAsync(hc, ctr, sizeof hc, cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    const size_t nf = (size_t)(hc[3] & 0xffffffffull);
+    std::vector<DetSeg> segs(nf);
+    if (nf) CU(cudaMemcpy(segs.data(), found, nf * sizeof(DetSeg), cudaMemcpyDeviceToHost));
+    // row order: the caller's contig order, then evaluation index; a replayed contig's second copy of a level goes
+    std::vector<DetSeg> keep;
+    keep.reserve(nf);
+    for (const DetSeg &d : segs)
+        if (d.contig >= 0 && d.contig < e->n && rank[(size_t)d.contig] >= 0) keep.push_back(d);
+    std::sort(keep.begin(), keep.end(), [&](const DetSeg &x, const DetSeg &y) {
+        const int64_t rx = rank[(size_t)x.contig], ry = rank[(size_t)y.contig];
+        return rx != ry ? rx < ry : (x.iter != y.iter ? x.iter < y.iter : x.start < y.start);
+    });
+    keep.erase(std::unique(keep.begin(), keep.end(), [](const DetSeg &x, const DetSeg &y) {
+        return x.contig == y.contig && x.iter == y.iter;
+    }), keep.end());
+    const size_t ns = keep.size();
+    DetSeg *dseg;
+    long long *dbytes, *doff;
+    if ((rc = outbuf(e, e->dt_seg, ns, &dseg)) || (rc = outbuf(e, e->dt_bytes, ns, &dbytes)) || (rc = outbuf(e, e->dt_off, ns, &doff)))
+        return rc;
+    if (ns) CU(cudaMemcpyAsync(dseg, keep.data(), ns * sizeof(DetSeg), cudaMemcpyHostToDevice, e->stream));
+    e->dt_seg_off.assign(ns + 1, 0);
+    if ((rc = details_rows(e, 0, (int64_t)ns, nullptr))) return rc;
+    std::vector<long long> nb(ns);
+    unsigned long long hc2[4];
+    CU(cudaMemcpyAsync(hc2, ctr, sizeof hc2, cudaMemcpyDeviceToHost, e->stream));
+    if (ns) CU(cudaMemcpyAsync(nb.data(), dbytes, ns * sizeof(long long), cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaEventRecord(e->ev[1], e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    if (hc2[2] & 0xffffffffull) {
+        set_err(e, "a gene score lies outside the exactly printable range |x| < 2^53");
+        return WFL_ERR_RANGE;
+    }
+    for (size_t s = 0; s < ns; ++s) e->dt_seg_off[s + 1] = e->dt_seg_off[s] + nb[s];
+    if (ns) CU(cudaMemcpyAsync(doff, e->dt_seg_off.data(), ns * sizeof(long long), cudaMemcpyHostToDevice, e->stream));
+    e->dt_rank_seg.assign((size_t)n_order + 1, 0);
+    size_t s = 0;
+    for (int64_t r = 0; r <= n_order; ++r) {
+        while (s < ns && rank[(size_t)keep[s].contig] < r) ++s;
+        e->dt_rank_seg[(size_t)r] = (int64_t)s;
+        if (bytes_before) bytes_before[r] = e->dt_seg_off[s];
+    }
+    CU(cudaStreamSynchronize(e->stream));
+    if (ms_kernels) CU(cudaEventElapsedTime(ms_kernels, e->ev[0], e->ev[1]));
+    e->dt_ready = true;
+    return e->dt_seg_off[ns];
+}
+
+int64_t wfl_details_text(wfl_engine *e, int64_t r0, int64_t r1, char *buf, int64_t capacity, float *ms_kernels,
+                         float *ms_d2h) {
+    if (!e) return WFL_ERR_ARG;
+    if (!e->dt_ready || !e->have_results) { set_err(e, "no prepared details: wfl_details_prepare after a details run"); return WFL_ERR_STATE; }
+    const int64_t n_order = (int64_t)e->dt_rank_seg.size() - 1;
+    if (r0 < 0 || r1 < r0 || r1 > n_order) { set_err(e, "bad range of the contig order"); return WFL_ERR_ARG; }
+    const int64_t s0 = e->dt_rank_seg[(size_t)r0], s1 = e->dt_rank_seg[(size_t)r1];
+    const int64_t total = e->dt_seg_off[(size_t)s1] - e->dt_seg_off[(size_t)s0];
+    if (!buf || capacity < total) return total;
+    CU(cudaSetDevice(e->device));
+    int rc;
+    char *text;
+    if ((rc = outbuf(e, e->dt_text, (size_t)total, &text))) return rc;
+    CU(cudaEventRecord(e->ev[0], e->stream));
+    if ((rc = details_rows(e, s0, s1, text))) return rc;
+    CU(cudaEventRecord(e->ev[1], e->stream));
+    if (total) CU(cudaMemcpyAsync(buf, text, (size_t)total, cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaEventRecord(e->ev[2], e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    if (ms_kernels) CU(cudaEventElapsedTime(ms_kernels, e->ev[0], e->ev[1]));
+    if (ms_d2h) CU(cudaEventElapsedTime(ms_d2h, e->ev[1], e->ev[2]));
+    return total;
+}
+
+int64_t wfl_debug_format_scores(wfl_engine *e, const double *x, int64_t n, char *text, int32_t *len) {
+    if (!e) return WFL_ERR_ARG;
+    if (n < 0 || (n && (!x || !text || !len))) { set_err(e, "bad arguments"); return WFL_ERR_ARG; }
+    CU(cudaSetDevice(e->device));
+    int rc;
+    const double *dx;
+    char *dt;
+    int *dl;
+    unsigned long long *ctr;
+    if ((rc = upload(e, e->dbg[2], x, (size_t)n, &dx)) || (rc = outbuf(e, e->dt_text, 24 * (size_t)n, &dt)) ||
+        (rc = outbuf(e, e->dbg[0], (size_t)n, &dl)) || (rc = outbuf(e, e->dt_ctr, 4, &ctr)))
+        return rc;
+    CU(cudaMemsetAsync(ctr, 0, 4 * sizeof(unsigned long long), e->stream));
+    if (n) launch_format3(dx, n, dt, dl, reinterpret_cast<unsigned int *>(ctr + 2), e->stream);
+    CU(cudaGetLastError());
+    unsigned long long hc[4];
+    CU(cudaMemcpyAsync(hc, ctr, sizeof hc, cudaMemcpyDeviceToHost, e->stream));
+    if (n) {
+        CU(cudaMemcpyAsync(text, dt, 24 * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
+        CU(cudaMemcpyAsync(len, dl, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, e->stream));
+    }
+    CU(cudaStreamSynchronize(e->stream));
+    if (hc[2] & 0xffffffffull) {
+        set_err(e, "%u value(s) outside the exactly printable range |x| < 2^53", (unsigned)(hc[2] & 0xffffffffull));
+        return WFL_ERR_RANGE;
+    }
+    return n;
 }
 
 }  // extern "C"

@@ -210,6 +210,47 @@ void launch_pipe_lift(const PipeArgs &a, int grid, cudaStream_t s);
 void launch_pipe_leftover(const PipeArgs &a, cudaStream_t s);
 int pipe_ctas_per_sm();
 
+// ---- --write-details text (wfl_details.cu) --------------------------------------------------------
+// One (contig, evaluation index) run of the details dump: entries [start, start + len).
+struct DetSeg {
+    long long start;
+    int len, contig, iter, pad;
+};
+
+struct DetTextArgs {
+    DevBatch b;
+    DevTax t;
+    DevParams P;
+    const int *anc;                // ancestor table (wfl_set_taxonomy): row l = l-th ancestor of every node
+    int anc_rows;
+    // the dump: contig, evaluation index, clade, raw locus index within the contig, score
+    const int32_t *dc, *di, *dc_clade, *dl;
+    const double *ds;
+    long long n_dump;
+    DetSeg *found;                 // segments kernel: every run of the dump, unordered ...
+    unsigned int *n_found;         // ... and their number
+    const DetSeg *seg;             // rows kernel: segments in row order
+    const int *list;               // segments to do: list[0, n_list), or null: [s0, s0 + n_list)
+    long long s0, n_list;
+    const char *cname;             // contig names by contig index: cname[cname_off[c], cname_off[c + 1])
+    const int64_t *cname_off;
+    const char *tname;             // clade names by node index
+    const int64_t *tname_off;
+    char *scratch;                 // `slice` bytes per warp
+    long long slice;
+    int *defer;                    // segments whose scratch exceeds the slice, their number and the largest need
+    unsigned int *n_defer;
+    unsigned long long *max_need;
+    long long *seg_bytes;          // length pass (text == null): bytes of every segment
+    char *text;                    // write pass: the text of the segments, segment si at text_off[si] - text_base
+    const long long *text_off;
+    long long text_base;
+    unsigned int *err;             // scores outside the formatter's exact range
+};
+void launch_details_segments(const DetTextArgs &a, cudaStream_t s);
+void launch_details_rows(const DetTextArgs &a, long long warps, cudaStream_t s);
+void launch_format3(const double *x, long long n, char *text, int *len, unsigned int *err, cudaStream_t s);
+
 // Compaction (K10): CSR of melded members in contig order + contig indices grouped by call.
 struct CompactArgs {
     int64_t n;

@@ -392,11 +392,8 @@ __global__ void __launch_bounds__(32, WFL_PIPE_CPSM) wfl_pipe_prepare(const Pipe
                         int cur = l_base[i + 1];
                         if (mt) {
                             int slot = cur + __popc(m & lt_mask());
-                            // python slice [h1 : h2+1] of a length-len array (:376-382)
-                            int s1 = max(0, hmin - lmin), e1 = min(len - 1, hmax - lmin) + 1;
-                            if (e1 < 0) e1 = max(0, e1 + len);
-                            s1 = min(s1, len);
-                            if (e1 < s1) e1 = s1;
+                            int s1, e1;
+                            hit_slice(hmin, hmax, lmin, len, s1, e1);
                             r_v[slot] = sc;
                             r_a[slot] = s1;
                             r_b[slot] = e1;

@@ -836,6 +836,16 @@ __device__ __noinline__ bool hit_matches(const DevParams &P, int hmin, int hmax,
     return ov >= P.p.min_overlap;
 }
 
+// site slice [s1, e1) a matched hit raises on a locus of length llen: the python slice [h1 : h2+1] of score_hit
+// (waafle_orgscorer.py:376-382), including the wrap of a negative stop; e1 == s1 for an empty slice
+__device__ __forceinline__ void hit_slice(int hmin, int hmax, int lmin, int llen, int &s1, int &e1) {
+    s1 = max(0, hmin - lmin);
+    e1 = min(llen - 1, hmax - lmin) + 1;
+    if (e1 < 0) e1 = max(0, e1 + llen);
+    s1 = min(s1, llen);
+    if (e1 < s1) e1 = s1;
+}
+
 
 }  // namespace
 }  // namespace wfl

@@ -28,7 +28,8 @@ EXPORTS = ["wfl_abi_version", "wfl_device_count", "wfl_create", "wfl_destroy", "
            "wfl_pack_results", "wfl_packed_results_layout", "wfl_debug_gene_scores", "wfl_host_alloc",
            "wfl_host_free", "wfl_parser_create", "wfl_parser_destroy", "wfl_parser_last_error", "wfl_parse_blast",
            "wfl_parse_distinct", "wfl_parse_fetch", "wfl_parser_times", "wfl_call_genes", "wfl_download_details", "wfl_parse_gff", "wfl_parse_gff_fetch",
-           "wfl_parser_call_genes", "wfl_parser_genes_fetch"]
+           "wfl_parser_call_genes", "wfl_parser_genes_fetch", "wfl_set_clade_names", "wfl_details_prepare",
+           "wfl_details_text", "wfl_debug_format_scores"]
 ABI_VERSION = 2
 _CUDA_TOUCHED = False   # this process has initialised CUDA through the library (a fork could not use it any more)
 
@@ -128,6 +129,15 @@ def load_library(path=None):
     lib.wfl_debug_gene_scores.argtypes = [ctypes.c_void_p, ctypes.c_int64, c_i32p, c_i32p, c_f64p,
                                           ctypes.c_int64]
     lib.wfl_debug_gene_scores.restype = ctypes.c_int64
+    lib.wfl_set_clade_names.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_char_p, c_i64p]
+    lib.wfl_details_prepare.argtypes = [ctypes.c_void_p, ctypes.c_int64, c_i32p, ctypes.c_char_p, c_i64p, c_i64p,
+                                        ctypes.POINTER(ctypes.c_float)]
+    lib.wfl_details_prepare.restype = ctypes.c_int64
+    lib.wfl_details_text.argtypes = [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p, ctypes.c_int64,
+                                     ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_float)]
+    lib.wfl_details_text.restype = ctypes.c_int64
+    lib.wfl_debug_format_scores.argtypes = [ctypes.c_void_p, c_f64p, ctypes.c_int64, ctypes.c_void_p, c_i32p]
+    lib.wfl_debug_format_scores.restype = ctypes.c_int64
     lib.wfl_host_alloc.argtypes = [ctypes.c_size_t, ctypes.POINTER(ctypes.c_void_p)]
     lib.wfl_host_free.argtypes = [ctypes.c_void_p]
     lib.wfl_host_free.restype = None
@@ -138,6 +148,14 @@ def load_library(path=None):
 
 def _ptr(a, ctype):
     return a.ctypes.data_as(ctypes.POINTER(ctype))
+
+
+def _name_blob(names):
+    """Names as one UTF-8 blob plus offsets [n + 1] (name i = blob[off[i]:off[i + 1]])."""
+    enc = [str(nm).encode() for nm in names]
+    off = np.zeros(len(enc) + 1, np.int64)
+    np.cumsum([len(b) for b in enc], out=off[1:])
+    return b"".join(enc), off
 
 
 def _as(a, dtype):
@@ -194,6 +212,8 @@ class Engine:
         self._pinned = None
         self._res_cache = {}
         self.n_systems = 0
+        self._clade_names = None        # names of the taxonomy's nodes, uploaded by the first details_text after set_taxonomy
+        self.details_times = {}
         if params is not None:
             self.set_params(params)
         if taxonomy is not None:
@@ -249,6 +269,7 @@ class Engine:
             self._h, len(parent), _ptr(parent, ctypes.c_int32), _ptr(depth, ctypes.c_int32),
             _ptr(leaf, ctypes.c_int32), _ptr(listed, ctypes.c_uint8),
             int(t["root_idx"]), int(t["unknown_idx"])))
+        self._clade_names = (list(tax.names), False) if getattr(tax, "names", None) is not None else None
 
     # ------------------------------------------------------------------
     def _cbatch(self, batch):
@@ -367,9 +388,11 @@ class Engine:
         self._check(self._lib.wfl_pack_results(self._h, ctypes.byref(p), ctypes.byref(nb), ctypes.byref(st)))
         return p.value, nb.value, st.value
 
-    def score_batch_details(self, batch):
+    def score_batch_details(self, batch, download=True):
         """--write-details: (results, details) where details = dict of arrays contig / iteration / clade / locus / score --
-        every gene score of every clade at every evaluated level (exact pipeline; see include/waafle_b200.h)."""
+        every gene score of every clade at every evaluated level (exact pipeline; see include/waafle_b200.h).  With
+        download=False the dump stays on the device (details_text reads it there), details is None and the engine keeps
+        recording details until set_option("details", 0)."""
         self.set_option("details", 0)
         self.set_option("exact", 1)
         self.score_batch(batch)
@@ -383,6 +406,13 @@ class Engine:
         for _ in range(4):
             self.set_option("details", cap)
             res = self.score_batch(batch)
+            if not download:
+                n = lib.wfl_download_details(self._h, None, None, None, None, None, 0)
+                self._check(min(int(n), 0))
+                if n <= cap:
+                    return res, None
+                cap = int(n) + 4096
+                continue
             d = dict(contig=np.empty(cap, np.int32), iteration=np.empty(cap, np.int32), clade=np.empty(cap, np.int32),
                      locus=np.empty(cap, np.int32), score=np.empty(cap, np.float64))
             n = lib.wfl_download_details(self._h, _ptr(d["contig"], ctypes.c_int32), _ptr(d["iteration"], ctypes.c_int32),
@@ -394,6 +424,57 @@ class Engine:
                 return res, {k: v[:int(n)] for k, v in d.items()}
             cap = int(n) + 4096
         raise EngineError("details dump keeps overflowing")
+
+    def details_text(self, order, contig_names, piece_bytes=256 << 20):
+        """The --write-details rows of the last score_batch_details run, built on the device, as bytes pieces of at most
+        `piece_bytes` each (a contig's rows are never split, so a contig larger than that is one piece).  `order`: contig
+        indices of the batch in output order; `contig_names`: the batch's contig names by index.  Needs a taxonomy with
+        names (taxonomy.Taxonomy).  Times of the last call land in `details_times` (ms)."""
+        if self._clade_names is None:
+            raise EngineError("details_text needs the node names of the taxonomy (set_taxonomy with a Taxonomy)")
+        names, sent = self._clade_names
+        if not sent:
+            blob, off = _name_blob(names)
+            self._check(self._lib.wfl_set_clade_names(self._h, len(names), blob, _ptr(off, ctypes.c_int64)))
+            self._clade_names = (names, True)
+        order = _as(order, np.int32)
+        blob, off = _name_blob(contig_names)
+        before = np.zeros(len(order) + 1, np.int64)
+        ms = ctypes.c_float()
+        total = self._lib.wfl_details_prepare(self._h, len(order), _ptr(order, ctypes.c_int32), blob,
+                                              _ptr(off, ctypes.c_int64), _ptr(before, ctypes.c_int64), ctypes.byref(ms))
+        self._check(min(int(total), 0))
+        times = dict(ms_length=ms.value, ms_text=0.0, ms_d2h=0.0, bytes=int(total), pieces=0)
+        self.details_times = times
+        r0, n = 0, len(order)
+        buf = None
+        while r0 < n:
+            # the longest run of contigs from r0 whose rows fit one piece (at least one contig)
+            r1 = max(r0 + 1, int(np.searchsorted(before, before[r0] + piece_bytes, side="right")) - 1)
+            size = int(before[r1] - before[r0])
+            if size:
+                if buf is None or len(buf) < size:
+                    buf = np.empty(max(size, min(int(total), int(piece_bytes))), np.uint8)
+                mk, md = ctypes.c_float(), ctypes.c_float()
+                got = self._lib.wfl_details_text(self._h, r0, r1, buf.ctypes.data, len(buf), ctypes.byref(mk), ctypes.byref(md))
+                self._check(min(int(got), 0))
+                if got != size:
+                    raise EngineError("details text: {} bytes, expected {}".format(got, size))
+                times["ms_text"] += mk.value
+                times["ms_d2h"] += md.value
+                times["pieces"] += 1
+                yield buf[:size].tobytes()
+            r0 = r1
+
+    def debug_format_scores(self, x):
+        """The details table's "{:.3f}" of every value of `x` (test hook); raises EngineError outside |x| < 2^53."""
+        x = _as(x, np.float64)
+        text = np.zeros(24 * max(1, len(x)), np.uint8)
+        lens = np.zeros(max(1, len(x)), np.int32)
+        self._check(min(int(self._lib.wfl_debug_format_scores(self._h, _ptr(x, ctypes.c_double), len(x), text.ctypes.data,
+                                                                _ptr(lens, ctypes.c_int32))), 0))
+        raw = text.tobytes()
+        return [raw[24 * i:24 * i + int(lens[i])].decode() for i in range(len(x))]
 
     def stats(self):
         s = CStats()

@@ -83,11 +83,6 @@ def streamed(args):
     return args.devices is not None or args.stream_mb > 0
 
 
-def check_flags(args):
-    if args.write_details and streamed(args):
-        die("--write-details needs the single-call path (no --devices / --stream-mb)")
-
-
 def params_from_args(args, n_systems):
     return OrgscorerParams.from_args(args, n_systems=n_systems)
 
@@ -142,7 +137,6 @@ def score_in_chunks(engine, batch, chunk):
 
 def main(argv=None):
     args = get_args(argv)
-    check_flags(args)
     say("Loading taxonomy.")
     tax = taxonomy.Taxonomy(args.taxonomy)
     say("Initializing contigs.")
@@ -184,10 +178,9 @@ def analyze(args, tax, contig_lengths, loci, hits=None):
     engine = Engine(args.device, params, tax)
     if args.exact_scores:
         engine.set_option("exact", 1)
-    det = None
     if args.write_details:
         # OS:931-937: every clade's gene scores at every evaluated level (the exact pipeline records them)
-        res, det = engine.score_batch_details(batch)
+        res, _ = engine.score_batch_details(batch, download=False)
     else:
         res = score_in_chunks(engine, batch, args.chunk_contigs)
     if not args.quiet:
@@ -195,12 +188,11 @@ def analyze(args, tax, contig_lengths, loci, hits=None):
         say("  scored {:,} contigs / {:,} hits on cuda:{} ({:.1f} ms in kernels; {:,} contigs on the exact pipeline, "
             "{:,} workspace replays)".format(batch.n_contigs, batch.n_hits, args.device, st["ms_kernels"],
                                              st["fallback_contigs"], st["workspace_retries"]))
+    if args.write_details:
+        from .streaming import details_order
+        writer.write_details_file(os.path.join(args.outdir, args.basename + ".details.tsv.gz"),
+                                  engine.details_text(details_order(batch, hits, contig_lengths), batch.contig_names))
     engine.close()
-    if det is not None:
-        from .streaming import chunk_contigs
-        index = {nm: k for k, nm in enumerate(batch.contig_names)}
-        order = [index[nm] for nm in chunk_contigs(hits, contig_lengths) if nm in index]   # blastout order (OS:944)
-        writer.write_details_file(os.path.join(args.outdir, args.basename + ".details.tsv.gz"), batch, tax, params, res, det, order)
     records = writer.build_records(batch, loci, hits, tax, res)
     writer.write_main_output_files(records, args.outdir, args.basename)
     say("Finished successfully.")

@@ -43,7 +43,6 @@ def gene_thresholds(args):
 
 def main(argv=None):
     args = get_args(argv)
-    orgscorer.check_flags(args)
     say("Loading taxonomy.")
     tax = taxonomy.Taxonomy(args.taxonomy)
     say("Initializing contigs.")

@@ -184,6 +184,12 @@ def chunk_contigs(hits, contig_lengths):
     return list(q[starts])
 
 
+def details_order(batch, hits, contig_lengths):
+    """Indices of the batch's contigs in blastout order: the row order of the details table (OS:944)."""
+    index = {nm: k for k, nm in enumerate(batch.contig_names)}
+    return [index[nm] for nm in dict.fromkeys(chunk_contigs(hits, contig_lengths)) if nm in index]
+
+
 def pack_chunk(names, contig_lengths, loci_index, hits, tax):
     """packing.pack restricted to the contigs `names` (FASTA-known ones); loci rows refer to the FULL locus table."""
     known = [nm for nm in dict.fromkeys(names) if nm in contig_lengths]
@@ -313,9 +319,10 @@ class ChunkScorer:
             calls = genecaller.call_genes(hits, *genes, device=self.device)[:5]
         return hits, calls
 
-    def score(self, names, hits, loci=None):
+    def score(self, names, hits, loci=None, details=None):
         """records of the contigs `names` given their parsed hits (possibly none); `loci`: the chunk's own LocusTable
-        (gene calls) instead of the rows of the loci index."""
+        (gene calls) instead of the rows of the loci index; `details`: path of the chunk's details shard (rows without
+        the header, blastout order) to write."""
         if hits.sysmask is None:
             die("more than 32 annotation systems in the subject headers")
         taxa = hits.distinct_taxa()
@@ -342,7 +349,12 @@ class ChunkScorer:
             if tax_changed:
                 self.engine.set_taxonomy(self.tax)
         self.n_systems = n_sys
-        res = self.engine.score_batch(batch)
+        if details is None:
+            res = self.engine.score_batch(batch)
+        else:
+            res, _ = self.engine.score_batch_details(batch, download=False)
+            writer.write_details_file(details, self.engine.details_text(details_order(batch, hits, self.contig_lengths),
+                                                                        batch.contig_names), header=False)
         st = self.engine.stats()
         self.stats["contigs"] += batch.n_contigs
         self.stats["hits"] += batch.n_hits
@@ -380,7 +392,8 @@ def _worker(wid, device, path, tasks, results, shard_dir, args, tax, contig_leng
                 else:
                     hits = scorer.parse(text)
                 names = chunk_contigs(hits, contig_lengths)
-                records, scored = scorer.score(names, hits, loci)
+                records, scored = scorer.score(names, hits, loci,
+                                               details=prefix + ".details.gz" if args.write_details else None)
                 write_shard(records, prefix)
                 results.put(("chunk", cid, prefix, list(scored), None))
         results.put(("done", wid, None, None, dict(scorer.stats, device=device)))
@@ -455,6 +468,9 @@ def run_streaming(args, tax, contig_lengths, loci, params_factory, devices, chun
             stats["rest"] = dict(scorer.stats, device=devices[0])
             scorer.close()
         merge_shards([prefixes[k] for k in sorted(prefixes)], args.outdir, args.basename)
+        if args.write_details:   # the contigs without hits ("rest") are never evaluated and have no rows (OS:959)
+            writer.concat_details_shards(os.path.join(args.outdir, args.basename + ".details.tsv.gz"),
+                                         [prefixes[k] + ".details.gz" for k in range(len(chunks))])
         if isinstance(loci_index, ChunkGenes) and loci_index.gff is not None:
             concat_gff_shards([prefixes[k] + ".gff" for k in range(len(chunks))], loci_index.gff)
     finally:

@@ -6,7 +6,11 @@ encodings (OS:750-764, 793-800), same float formatting and `--` for empty cells
 (waafle/utils.py:137-139), rows sorted by contig name (OS:838).
 """
 
+import collections
+import concurrent.futures
 import os
+import shutil
+import zlib
 
 import numpy as np
 
@@ -154,120 +158,51 @@ def write_main_output_files(records, outdir, basename):
 # ---------------------------------------------------------------------------------------------------------------
 
 DETAILS_FORMAT = ["contig_name", "iteration", "clade", "gene_scores", "gene_spans"]   # OS:116-122
-C_PRECISION = 3                                                                       # OS:59
-C_DELIM3 = ":"                                                                        # OS:66
+DETAILS_LEVEL = 6             # zlib's default level: about twice as fast as gzip's 9 for a few % more bytes
+DETAILS_BLOCK = 16 << 20      # text per gzip member: the unit of parallel compression
 
 
-def _calc_overlap(a1, a2, b1, b2):
-    """UT:487-500."""
-    a1, a2 = sorted([a1, a2])
-    b1, b2 = sorted([b1, b2])
-    if b1 > a2 or a1 > b2:
-        return 0
-    _, inleft, inright, _ = sorted([a1, a2, b1, b2])
-    return (inright - inleft + 1) / float(min(a2 - a1 + 1, b2 - b1 + 1))
+def gzip_member(data, level=DETAILS_LEVEL):
+    """`data` as one complete gzip member."""
+    z = zlib.compressobj(level, zlib.DEFLATED, 31)
+    return z.compress(data) + z.flush()
 
 
-def _contig_records(batch, params, c):
-    """(retained locus rows, [(taxon index, retained locus k, python slice start, stop)]) of contig c: the hits that
-    attach_hits (OS:359-369) scores and the site slices score_hit (OS:371-382) raises above zero (start == stop for a hit
-    that creates the site array but leaves it at zero)."""
-    l0, l1 = int(batch.locus_off[c]), int(batch.locus_off[c + 1])
-    kept = [j for j in range(l0, l1)
-            if abs(int(batch.locus_end[j]) - int(batch.locus_start[j])) + 1 >= params.min_gene_length]
-    recs = []
-    for h in range(int(batch.hit_off[c]), int(batch.hit_off[c + 1])):
-        if not batch.hit_scov[h] >= params.min_scov:
-            continue
-        for k, j in enumerate(kept):
-            if params.stranded and int(batch.hit_strand[h]) != int(batch.locus_strand[j]):
-                continue
-            qs, qe = int(batch.hit_qstart[h]), int(batch.hit_qend[h])
-            ls, le = int(batch.locus_start[j]), int(batch.locus_end[j])
-            if not _calc_overlap(qs, qe, ls, le) >= params.min_overlap:
-                continue
-            lo, n = min(ls, le), abs(le - ls) + 1
-            h1 = max(0, min(qs, qe) - lo)
-            h2 = min(n - 1, max(qs, qe) - lo)
-            a, b, _ = slice(h1, h2 + 1).indices(n)   # python slice semantics incl. the wrap of a negative stop
-            if not (b > a and batch.hit_score[h] > 0.0):
-                b = a                                # the site array exists but this hit leaves it at zero
-            recs.append((int(batch.hit_taxon[h]), k, a, b))
-    return kept, recs
+def write_gzip_members(fh, pieces, threads=None):
+    """Concatenated gzip members of the byte strings `pieces` (cut into DETAILS_BLOCK blocks), compressed in a thread pool
+    (zlib releases the GIL) while the next pieces are produced, written to the binary handle `fh` in order.  A
+    multi-member file reads back with gzip.open like any gzip file."""
+    threads = threads or min(32, os.cpu_count() or 1)
+    pending = collections.deque()
+    with concurrent.futures.ThreadPoolExecutor(threads) as pool:
+        for piece in pieces:
+            view = memoryview(piece)
+            for i in range(0, len(view), DETAILS_BLOCK):
+                pending.append(pool.submit(gzip_member, view[i:i + DETAILS_BLOCK]))
+            while len(pending) > 2 * threads:
+                fh.write(pending.popleft().result())
+        while pending:
+            fh.write(pending.popleft().result())
+    return threads
 
 
-def _spans_field(runs):
-    """make_gene_spans_field (OS:773-791) of one site array given its non-zero runs [a, b) (0-based): the 1-based first and
-    last site of every run of at least two sites."""
-    out = []
-    for a, b in runs:
-        if b - a >= 2:
-            out += [a + 1, b]
-    return C_DELIM3.join(str(k) for k in out)
+def details_header():
+    return ("\t".join(k.upper() for k in DETAILS_FORMAT) + "\n").encode()
 
 
-def write_details_file(path, batch, taxonomy, params, res, det, contig_order):
-    """<basename>.details.tsv.gz (OS:931-937, 802-812): per contig (blastout order), evaluated level and clade (ascending
-    name -- the reference walks a set) the clade's gene scores (3 decimals) and the non-zero spans of its site arrays.
-    `det`: the engine's dump (Engine.score_batch_details).  Iterations are numbered like upstream: 1, 1, 2, 3, ...
-    (OS:566-579 writes the level after the first raise before incrementing)."""
-    import gzip
-    names = taxonomy.names
-    parent = taxonomy.tables()["parent"]
-    order = np.lexsort((det["locus"], det["clade"], det["iteration"], det["contig"]))
-    dc, di, dl, dk, ds = (det[k][order] for k in ("contig", "iteration", "clade", "locus", "score"))
-    starts = np.flatnonzero(np.r_[True, dc[1:] != dc[:-1]]) if len(dc) else np.zeros(0, np.int64)
-    seg = {int(dc[s]): (int(s), int(e)) for s, e in zip(starts, np.r_[starts[1:], len(dc)])}
-    jump = int(params.jump_taxonomy)
-    with gzip.open(path, "wt") as fh:
-        write_row([k.upper() for k in DETAILS_FORMAT], fh)
-        for c in contig_order:
-            if c not in seg:
-                continue   # no hits, or every locus ignored: the contig is never evaluated (OS:959)
-            s, e = seg[c]
-            kept, recs = _contig_records(batch, params, c)
-            l0 = int(batch.locus_off[c])
-            slot = {j - l0: k for k, j in enumerate(kept)}
-            G = len(kept)
-            # clade of every record at the current level
-            cur = [t for t, _, _, _ in recs]
-            for _ in range(jump):
-                cur = [int(parent[t]) for t in cur]
-            it = 0
-            p = s
-            while p < e:
-                q = p
-                while q < e and di[q] == di[p]:
-                    q += 1
-                level = int(di[p])
-                while it < level:   # raise_taxonomy (OS:431-445)
-                    cur = [int(parent[t]) for t in cur]
-                    it += 1
-                rows, spans = {}, {}
-                for x in range(p, q):
-                    rows.setdefault(int(dl[x]), [0.0] * G)[slot[int(dk[x])]] = float(ds[x])
-                for (t0, k, a, b), t in zip(recs, cur):
-                    spans.setdefault(t, {}).setdefault(k, []).append((a, b))
-                for t in sorted(rows):
-                    cells = []
-                    for k in range(G):
-                        if k not in spans.get(t, {}):
-                            cells.append(C_MISSING_ANNOTATION)   # no site array for this clade / locus (OS:776-781)
-                            continue
-                        iv = sorted(x for x in spans[t][k] if x[1] > x[0])
-                        if not iv:
-                            cells.append("")
-                            continue
-                        runs, (ca, cb) = [], iv[0]
-                        for a, b in iv[1:]:
-                            if a <= cb:
-                                cb = max(cb, b)
-                            else:
-                                runs.append((ca, cb))
-                                ca, cb = a, b
-                        runs.append((ca, cb))
-                        cells.append(_spans_field(runs))
-                    write_row([format_field(v) for v in (
-                        batch.contig_names[c], max(1, level), names[t],
-                        "|".join("{:.{p}f}".format(v, p=C_PRECISION) for v in rows[t]), "|".join(cells))], fh)
-                p = q
+def write_details_file(path, pieces, header=True):
+    """<basename>.details.tsv.gz (OS:931-937, 802-812): the header row, then the rows the engine built on the device
+    (Engine.details_text), as concatenated gzip members.  header=False writes a shard of a streamed run."""
+    with open(path, "wb") as fh:
+        if header:
+            fh.write(gzip_member(details_header()))
+        return write_gzip_members(fh, pieces)
+
+
+def concat_details_shards(path, shards):
+    """The header member, then the details shards of a streamed run in chunk (= blastout) order."""
+    with open(path, "wb") as dst:
+        dst.write(gzip_member(details_header()))
+        for shard in shards:
+            with open(shard, "rb") as src:
+                shutil.copyfileobj(src, dst)
