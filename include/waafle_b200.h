@@ -38,7 +38,8 @@ typedef enum {
     WFL_ERR_STATE = -3,     /* params / taxonomy / batch not set             */
     WFL_ERR_CAPACITY = -4,  /* caller-provided output buffer too small       */
     WFL_ERR_RUNAWAY = -5,   /* >100 taxonomy lifts (reference: wu.die, waafle_orgscorer.py:580-581) */
-    WFL_ERR_RANGE = -6      /* a score outside the range the details formatter prints exactly (|x| < 2^53)  */
+    WFL_ERR_RANGE = -6,     /* a score outside the range the details formatter prints exactly (|x| < 2^53)  */
+    WFL_ERR_DATA = -7       /* compressed input that fails validation (wfl_inflate_bgzf)  */
 } wfl_status;
 
 /* Engine-relevant CLI flags (waafle_orgscorer.py:188-296, waafle_genecaller.py:83-101;
@@ -228,8 +229,24 @@ typedef struct wfl_parser wfl_parser;
 int  wfl_parser_create(int device, wfl_parser **out);
 void wfl_parser_destroy(wfl_parser *p);
 const char *wfl_parser_last_error(const wfl_parser *p);
-/* returns the number of rows or a negative wfl_status */
+/* returns the number of rows or a negative wfl_status; = an upload of the text followed by wfl_parse_blast_resident */
 int64_t wfl_parse_blast(wfl_parser *p, const char *text, int64_t n_bytes, int32_t *flagged, int64_t *first_flagged);
+/* Parse bytes [off, off + n_bytes) of the text already resident on the parser (the last wfl_parse_blast upload or
+ * wfl_inflate_bgzf).  Same results as wfl_parse_blast on those bytes: ss_off / q_off and the distinct-name offsets are
+ * relative to `off`.  WFL_ERR_ARG for a range outside the resident text. */
+int64_t wfl_parse_blast_resident(wfl_parser *p, int64_t off, int64_t n_bytes, int32_t *flagged, int64_t *first_flagged);
+/* Copy resident text [off, off + n_bytes) to dst (the host side's names are slices of it). */
+int  wfl_parser_text(wfl_parser *p, int64_t off, int64_t n_bytes, char *dst);
+/* BGZF (bgzip's gzip variant) inflated on the device into the parser's resident text.  `comp`: the compressed bytes;
+ * `members`: [n_members][5] = offset of the raw DEFLATE payload in comp, its length, ISIZE, CRC-32 and the member's
+ * output offset (an exclusive prefix sum of ISIZE; members of at most 64 KB).  Every member is decoded and checked
+ * (stored / fixed / dynamic blocks; bounds of the payload, code-length sets, symbols 286-287 and distances 30-31, no
+ * distance before the member's start, exactly ISIZE bytes, the CRC-32).  Returns the text length; WFL_ERR_DATA when a
+ * member fails (*bad_member = the first one, else -1: the caller reads the file on the host), WFL_ERR_ARG for a member
+ * table that does not fit `comp` or does not tile the text.  ms_* (NULL = skip): CUDA-event times of the upload and of
+ * the inflate kernel. */
+int64_t wfl_inflate_bgzf(wfl_parser *p, const uint8_t *comp, int64_t comp_len, const int64_t *members, int64_t n_members,
+                         int64_t *bad_member, float *ms_h2d, float *ms_kernel);
 /* distinct-name sets of the last parse: kind 0 = taxa (2^20 slots), 1 = annotation systems (64 slots); hash[s] != 0 marks
  * an occupied slot and (off[s], len[s]) is one occurrence of its name in the text */
 int  wfl_parse_distinct(wfl_parser *p, int kind, uint64_t *hash, int64_t *off, int32_t *len, int32_t slots);

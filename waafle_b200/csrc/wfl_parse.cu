@@ -449,7 +449,7 @@ void wfl_parser_destroy(wfl_parser *p) {
     if (!p) return;
     cudaSetDevice(p->device);
     PBuf *all[] = {&p->text, &p->tiles, &p->rows, &p->tax_hash, &p->tax_off, &p->tax_len, &p->sys_hash,
-                   &p->sys_off, &p->sys_len, &p->counters, &p->perm};
+                   &p->sys_off, &p->sys_len, &p->counters, &p->perm, &p->comp, &p->mtab};
     for (PBuf *b : all) if (b->p) cudaFree(b->p);
     for (auto &b : p->col) if (b.p) cudaFree(b.p);
     for (auto &b : p->gcol) if (b.p) cudaFree(b.p);
@@ -461,12 +461,27 @@ void wfl_parser_destroy(wfl_parser *p) {
 
 const char *wfl_parser_last_error(const wfl_parser *p) { return p ? p->err : "null parser"; }
 
-/* Ship `n_bytes` of blastout text (whole rows; the caller owns the buffer) and parse it on the device.  Returns the
- * number of rows (>= 0) or a negative wfl_status; *flagged = rows the device parser cannot reproduce exactly (then
- * *first_flagged is the first such row and the caller must use the CPU reader). */
-int64_t wfl_parse_blast(wfl_parser *p, const char *text, int64_t n_bytes, int32_t *flagged, int64_t *first_flagged) {
-    if (!p || (!text && n_bytes) || n_bytes < 0) return WFL_ERR_ARG;
-    PCU(cudaSetDevice(p->device));
+}  // extern "C"
+
+namespace {
+
+// the parse buffers whose size the text alone decides (a no-op when they are large enough)
+int parse_buffers(wfl_parser *p, long long n_bytes) {
+    int rc;
+    const long long n_tiles = (n_bytes + TILE - 1) / TILE;
+    if ((rc = pensure(p, p->tiles, (size_t)(n_tiles + 1) * 8)) || (rc = pensure(p, p->tax_hash, (size_t)TAX_SLOTS * 8)) ||
+        (rc = pensure(p, p->tax_off, (size_t)TAX_SLOTS * 8)) || (rc = pensure(p, p->tax_len, (size_t)TAX_SLOTS * 4)) ||
+        (rc = pensure(p, p->sys_hash, SYS_SLOTS * 8)) || (rc = pensure(p, p->sys_off, SYS_SLOTS * 8)) ||
+        (rc = pensure(p, p->sys_len, SYS_SLOTS * 4)) || (rc = pensure(p, p->counters, 16)) ||
+        (rc = pensure(p, p->perm, SYS_SLOTS * 4)))
+        return rc;
+    return WFL_OK;
+}
+
+// parse bytes [off, off + n_bytes) of the resident text.  `host_text`: the same bytes on the host when the caller has just
+// uploaded them (it recorded ev[0] before the copy), else NULL: the one byte the host needs then comes from the device.
+int64_t parse_resident(wfl_parser *p, long long off, long long n_bytes, int32_t *flagged, int64_t *first_flagged,
+                       const char *host_text) {
     p->n_bytes = n_bytes;
     p->n_rows = 0;
     p->blast_ok = p->genes_ok = false;
@@ -478,30 +493,25 @@ int64_t wfl_parse_blast(wfl_parser *p, const char *text, int64_t n_bytes, int32_
     }
     int rc;
     const long long n_tiles = (n_bytes + TILE - 1) / TILE;
-    if ((rc = pensure(p, p->text, (size_t)n_bytes + 64)) || (rc = pensure(p, p->tiles, (size_t)(n_tiles + 1) * 8))) return rc;
-    if ((rc = pensure(p, p->tax_hash, (size_t)TAX_SLOTS * 8)) || (rc = pensure(p, p->tax_off, (size_t)TAX_SLOTS * 8)) ||
-        (rc = pensure(p, p->tax_len, (size_t)TAX_SLOTS * 4)) || (rc = pensure(p, p->sys_hash, SYS_SLOTS * 8)) ||
-        (rc = pensure(p, p->sys_off, SYS_SLOTS * 8)) || (rc = pensure(p, p->sys_len, SYS_SLOTS * 4)) ||
-        (rc = pensure(p, p->counters, 16)) || (rc = pensure(p, p->perm, SYS_SLOTS * 4)))
-        return rc;
-    PCU(cudaEventRecord(p->ev[0], p->stream));
-    PCU(cudaMemcpyAsync(p->text.p, text, (size_t)n_bytes, cudaMemcpyHostToDevice, p->stream));
+    if ((rc = parse_buffers(p, n_bytes))) return rc;
     PCU(cudaEventRecord(p->ev[1], p->stream));
     PCU(cudaMemsetAsync(p->tax_hash.p, 0, (size_t)TAX_SLOTS * 8, p->stream));
     PCU(cudaMemsetAsync(p->sys_hash.p, 0, SYS_SLOTS * 8, p->stream));
     const int init[4] = {0, 0, 0, 2147483647};
     PCU(cudaMemcpyAsync(p->counters.p, init, sizeof init, cudaMemcpyHostToDevice, p->stream));
     ParseArgs a{};
-    a.text = static_cast<const char *>(p->text.p);
+    a.text = static_cast<const char *>(p->text.p) + off;
     a.n_bytes = n_bytes;
     a.tile_count = static_cast<long long *>(p->tiles.p);
     a.n_tiles = n_tiles;
     wfl_parse_lines_count<<<(unsigned)n_tiles, TPB, 0, p->stream>>>(a);
     wfl_parse_lines_scan<<<1, 1024, 0, p->stream>>>(a);
     long long n_newlines = 0;
+    char last = host_text ? host_text[n_bytes - 1] : 0;
     PCU(cudaMemcpyAsync(&n_newlines, a.tile_count + n_tiles, 8, cudaMemcpyDeviceToHost, p->stream));
+    if (!host_text) PCU(cudaMemcpyAsync(&last, a.text + n_bytes - 1, 1, cudaMemcpyDeviceToHost, p->stream));
     PCU(cudaStreamSynchronize(p->stream));
-    const bool unterminated = text[n_bytes - 1] != '\n';
+    const bool unterminated = last != '\n';
     const long long n_rows = n_newlines + (unterminated ? 1 : 0);
     p->n_rows = n_rows;
     if ((rc = pensure(p, p->rows, (size_t)(n_rows + 2) * 8))) return rc;
@@ -532,12 +542,51 @@ int64_t wfl_parse_blast(wfl_parser *p, const char *text, int64_t n_bytes, int32_
     int counters[4];
     PCU(cudaMemcpyAsync(counters, p->counters.p, sizeof counters, cudaMemcpyDeviceToHost, p->stream));
     PCU(cudaStreamSynchronize(p->stream));
-    PCU(cudaEventElapsedTime(&p->ms_h2d, p->ev[0], p->ev[1]));
+    p->ms_h2d = 0;
+    if (host_text) PCU(cudaEventElapsedTime(&p->ms_h2d, p->ev[0], p->ev[1]));
     PCU(cudaEventElapsedTime(&p->ms_kernels, p->ev[1], p->ev[2]));
     if (flagged) *flagged = counters[2];
     if (first_flagged) *first_flagged = counters[2] ? counters[3] : -1;
     p->blast_ok = counters[2] == 0;
     return n_rows;
+}
+
+}  // namespace
+
+extern "C" {
+
+/* Ship `n_bytes` of blastout text (whole rows; the caller owns the buffer) and parse it on the device.  Returns the
+ * number of rows (>= 0) or a negative wfl_status; *flagged = rows the device parser cannot reproduce exactly (then
+ * *first_flagged is the first such row and the caller must use the CPU reader). */
+int64_t wfl_parse_blast(wfl_parser *p, const char *text, int64_t n_bytes, int32_t *flagged, int64_t *first_flagged) {
+    if (!p || (!text && n_bytes) || n_bytes < 0) return WFL_ERR_ARG;
+    PCU(cudaSetDevice(p->device));
+    p->text_bytes = 0;
+    if (n_bytes > 0) {
+        int rc;
+        if ((rc = pensure(p, p->text, (size_t)n_bytes + 64)) || (rc = parse_buffers(p, n_bytes))) return rc;
+        PCU(cudaEventRecord(p->ev[0], p->stream));
+        PCU(cudaMemcpyAsync(p->text.p, text, (size_t)n_bytes, cudaMemcpyHostToDevice, p->stream));
+        p->text_bytes = n_bytes;
+    }
+    return parse_resident(p, 0, n_bytes, flagged, first_flagged, text);
+}
+
+/* Parse bytes [off, off + n_bytes) of the resident text (an upload or a BGZF inflate); offsets relative to `off`. */
+int64_t wfl_parse_blast_resident(wfl_parser *p, int64_t off, int64_t n_bytes, int32_t *flagged, int64_t *first_flagged) {
+    if (!p || off < 0 || n_bytes < 0 || off > p->text_bytes - n_bytes) return WFL_ERR_ARG;
+    PCU(cudaSetDevice(p->device));
+    return parse_resident(p, off, n_bytes, flagged, first_flagged, nullptr);
+}
+
+/* Resident text [off, off + n_bytes) to the host. */
+int wfl_parser_text(wfl_parser *p, int64_t off, int64_t n_bytes, char *dst) {
+    if (!p || off < 0 || n_bytes < 0 || off > p->text_bytes - n_bytes || (!dst && n_bytes)) return WFL_ERR_ARG;
+    if (n_bytes == 0) return WFL_OK;
+    PCU(cudaSetDevice(p->device));
+    PCU(cudaMemcpyAsync(dst, static_cast<const char *>(p->text.p) + off, (size_t)n_bytes, cudaMemcpyDeviceToHost, p->stream));
+    PCU(cudaStreamSynchronize(p->stream));
+    return WFL_OK;
 }
 
 /* The distinct-name sets of the last parse: kind 0 = taxa (2^20 slots), 1 = annotation systems (64 slots).  hash[s] != 0
@@ -592,6 +641,7 @@ int64_t wfl_parse_gff(wfl_parser *p, const char *text, int64_t n_bytes, int32_t 
     if (!p || (!text && n_bytes) || n_bytes < 0) return WFL_ERR_ARG;
     PCU(cudaSetDevice(p->device));
     p->gff_rows = 0;
+    p->text_bytes = 0;   // the text buffer now holds the GFF
     if (flagged) *flagged = 0;
     if (first_flagged) *first_flagged = -1;
     if (n_bytes == 0) return 0;

@@ -27,6 +27,8 @@ struct wfl_parser {
     long long gff_rows = 0;
     wfl::PBuf text, tiles, rows, col[13], tax_hash, tax_off, tax_len, sys_hash, sys_off, sys_len, counters, perm;
     long long n_rows = 0, n_bytes = 0;
+    long long text_bytes = 0;         // valid bytes of `text`: the last upload or BGZF inflate
+    wfl::PBuf comp, mtab;             // compressed bytes and member table of the last wfl_inflate_bgzf
     bool blast_ok = false;            // col[] holds the last wfl_parse_blast, which flagged no row
     wfl::PBuf gc_pool;                // gene-call scratch and the dense gene arrays of the last wfl_parser_call_genes
     bool genes_ok = false;

@@ -27,7 +27,7 @@ EXPORTS = ["wfl_abi_version", "wfl_device_count", "wfl_create", "wfl_destroy", "
            "wfl_upload_packed", "wfl_run_resident", "wfl_download_results", "wfl_get_stats", "wfl_set_option",
            "wfl_pack_results", "wfl_packed_results_layout", "wfl_debug_gene_scores", "wfl_host_alloc",
            "wfl_host_free", "wfl_parser_create", "wfl_parser_destroy", "wfl_parser_last_error", "wfl_parse_blast",
-           "wfl_parse_distinct", "wfl_parse_fetch", "wfl_parser_times", "wfl_call_genes", "wfl_download_details", "wfl_parse_gff", "wfl_parse_gff_fetch",
+           "wfl_parse_blast_resident", "wfl_parser_text", "wfl_inflate_bgzf", "wfl_parse_distinct", "wfl_parse_fetch", "wfl_parser_times", "wfl_call_genes", "wfl_download_details", "wfl_parse_gff", "wfl_parse_gff_fetch",
            "wfl_parser_call_genes", "wfl_parser_genes_fetch", "wfl_set_clade_names", "wfl_details_prepare",
            "wfl_details_text", "wfl_debug_format_scores"]
 ABI_VERSION = 2

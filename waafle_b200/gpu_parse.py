@@ -30,6 +30,13 @@ def _lib():
         lib.wfl_parser_last_error.restype = ctypes.c_char_p
         lib.wfl_parse_blast.argtypes = [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_int64, P(ctypes.c_int32), P(ctypes.c_int64)]
         lib.wfl_parse_blast.restype = ctypes.c_int64
+        lib.wfl_parse_blast_resident.argtypes = [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, P(ctypes.c_int32),
+                                                 P(ctypes.c_int64)]
+        lib.wfl_parse_blast_resident.restype = ctypes.c_int64
+        lib.wfl_parser_text.argtypes = [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p]
+        lib.wfl_inflate_bgzf.argtypes = [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_int64,
+                                         P(ctypes.c_int64), P(ctypes.c_float), P(ctypes.c_float)]
+        lib.wfl_inflate_bgzf.restype = ctypes.c_int64
         lib.wfl_parse_distinct.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                            ctypes.c_int32]
         lib.wfl_parse_fetch.argtypes = [ctypes.c_void_p] + [ctypes.c_void_p] * 13
@@ -43,6 +50,14 @@ def _lib():
         lib.wfl_parser_genes_fetch.argtypes = [ctypes.c_void_p] + [ctypes.c_void_p] * 4
         _ready = True
     return lib
+
+
+class InflateError(EngineError):
+    """A BGZF member failed validation on the device (`member`: the first such member of the table)."""
+
+    def __init__(self, member):
+        super().__init__("BGZF member {} failed validation on the device".format(member))
+        self.member = member
 
 
 class _TextNames:
@@ -90,17 +105,60 @@ class BlastParser:
     def parse(self, text):
         """`text`: bytes of a whole blastout file (or of whole rows of it).  Returns a parsers.HitTable, or None if some
         row needs the CPU reader."""
-        from . import parsers
         if not isinstance(text, (bytes, bytearray)):
             text = bytes(text)
         flagged, first = ctypes.c_int32(), ctypes.c_int64()
         if len(text.strip()) == 0:   # an empty parse on the device too, so that call_genes sees no blocks
-            self._check(self._lib.wfl_parse_blast(self._h, b"", 0, ctypes.byref(flagged), ctypes.byref(first)))
-            return parsers.hits_from_columns(*([[]] * 10))
+            text = b""
         n = self._lib.wfl_parse_blast(self._h, text, len(text), ctypes.byref(flagged), ctypes.byref(first))
+        return self._collect(text, n, flagged)
+
+    def inflate_bgzf(self, comp, members):
+        """Inflate BGZF bytes `comp` (member table `members`, compressed.bgzf_members) into the parser's resident text on
+        the device.  Returns the text length; raises InflateError when a member fails validation."""
+        members = np.ascontiguousarray(members, dtype=np.int64)
+        bad, h2d, kern = ctypes.c_int64(), ctypes.c_float(), ctypes.c_float()
+        n = self._lib.wfl_inflate_bgzf(self._h, bytes(comp), len(comp), members.ctypes.data_as(ctypes.c_void_p),
+                                       len(members), ctypes.byref(bad), ctypes.byref(h2d), ctypes.byref(kern))
+        if bad.value >= 0:
+            raise InflateError(int(bad.value))
+        self._check(n)
+        self.inflate_times = dict(ms_h2d=h2d.value, ms_inflate=kern.value, members=len(members), comp_bytes=len(comp),
+                                  text_bytes=int(n))
+        return int(n)
+
+    def text(self, off, n):
+        """Bytes [off, off + n) of the resident text (a bytearray, filled in place)."""
+        buf = bytearray(int(n))
+        dst = ctypes.addressof((ctypes.c_char * len(buf)).from_buffer(buf)) if len(buf) else None
+        self._check(self._lib.wfl_parser_text(self._h, int(off), int(n), dst))
+        return buf
+
+    def parse_bgzf(self, comp, members, own=None):
+        """Inflate BGZF bytes on the device and parse the text where it lies.  `own` = (offset, length): parse only that
+        byte range of the text (whole rows).  Returns the same HitTable as `parse` on the same text, or None if some row
+        needs the CPU reader (`text(*own)` then gives the rows); raises InflateError for a member that fails validation."""
+        size = self.inflate_bgzf(comp, members)
+        off, n = own if own is not None else (0, size)
+        text = self.text(off, n)
+        if len(text.strip()) == 0:
+            off, n = 0, 0
+        flagged, first = ctypes.c_int32(), ctypes.c_int64()
+        rows = self._lib.wfl_parse_blast_resident(self._h, off, n, ctypes.byref(flagged), ctypes.byref(first))
+        hits = self._collect(text if n else b"", rows, flagged)
+        if hits is not None:
+            self.times.update(self.inflate_times)
+        return hits
+
+    def _collect(self, text, n, flagged):
+        """The HitTable of the parse that returned `n` rows over host bytes `text` (None: a row needs the CPU reader)."""
+        from . import parsers
         self._check(n)
         if flagged.value:
             return None
+        if len(text) == 0:
+            self.times = dict(ms_h2d=0.0, ms_kernels=0.0, ms_d2h=0.0, rows=0, bytes=0)
+            return parsers.hits_from_columns(*([[]] * 10))
         n = int(n)
         # ---- the distinct names: taxa (2^20 slots) and annotation systems (64 slots) ----
         vp = lambda a: a.ctypes.data_as(ctypes.c_void_p)

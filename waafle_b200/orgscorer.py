@@ -164,8 +164,10 @@ def analyze(args, tax, contig_lengths, loci, hits=None):
         if not args.quiet:
             for w in sorted(k for k in stats if k != "rest"):
                 st = stats[w]
-                say("  worker {} on cuda:{}: {:,} contigs / {:,} hits in {} chunk(s) ({:.1f} ms in kernels)".format(
-                    w, st["device"], st["contigs"], st["hits"], st["chunks"], st["ms_kernels"]))
+                say("  worker {} on cuda:{}: {:,} contigs / {:,} hits in {} chunk(s) ({:.1f} ms in kernels{})".format(
+                    w, st["device"], st["contigs"], st["hits"], st["chunks"], st["ms_kernels"],
+                    "; {:,} BGZF members inflated on the device".format(st["inflated_members"])
+                    if st.get("inflated_members") else ""))
         say("Finished successfully.")
         return
     if hits is None:

@@ -20,7 +20,7 @@ try:   # Arrow's CSV reader and string kernels (multi-threaded, no per-row Pytho
 except Exception:   # pragma: no cover
     pa = pc = pacsv = None
 
-from .utils import die, try_open
+from .utils import die, say, try_open
 
 # UT:167-183
 BLAST_FIELDS = ["qseqid", "sseqid", "qlen", "slen", "length", "qstart", "qend", "sstart",
@@ -313,12 +313,29 @@ def _read_bytes(path):
 
 def _gpu_parse_blast(path, device, genes=None):
     """The blastout parsed on the GPU (None: the CPU reader must take the file).  `genes` = (min_overlap, min_gene_length,
-    min_scov): gene calls over the parsed columns before the parser goes, returned as (HitTable, genes)."""
-    from . import gpu_parse
-    text = _read_bytes(path)
+    min_scov): gene calls over the parsed columns before the parser goes, returned as (HitTable, genes).  A BGZF blastout
+    is inflated on the device (its compressed bytes cross PCIe, not the text); other compressed files are inflated on
+    the host.  A BGZF member that fails validation on the device sends the file to the CPU reader, which raises the error
+    Python's gzip raises on it."""
+    from . import compressed, gpu_parse
+    kind, members = compressed.classify(path)
+    if kind == compressed.BGZF:
+        with open(path, "rb") as fh:
+            comp = fh.read()
+    else:
+        text = _read_bytes(path)
     parser = gpu_parse.BlastParser(device)
     try:
-        hits = parser.parse(text)
+        if kind == compressed.BGZF:
+            try:
+                hits = parser.parse_bgzf(comp, members)
+                say("  blastout: BGZF, {:,} members inflated on cuda:{}".format(len(members), device))
+            except gpu_parse.InflateError as exc:
+                say("  blastout: BGZF member {} failed validation on cuda:{}; reading the file on the host".format(
+                    exc.member, device))
+                hits = None
+        else:
+            hits = parser.parse(text)
         calls = parser.call_genes(*genes) if genes is not None and hits is not None else None
     finally:
         parser.close()

@@ -49,66 +49,105 @@ def _first_query_change(buf, carry_name):
 def scan_blast_chunks(path, target_bytes):
     """[(offset, length)] covering the file; every range but the first starts at a row whose query name differs from the
     previous row's, and ranges are ~target_bytes long (a single contig's block is never split)."""
-    size = os.path.getsize(path)
-    chunks, start = [], 0
     with open(path, "rb") as fh:
-        while start < size:
-            want = start + target_bytes
-            if want >= size:
-                chunks.append((start, size - start))
+        return scan_text_chunks(fh, os.path.getsize(path), target_bytes)
+
+
+def scan_text_chunks(fh, size, target_bytes):
+    """scan_blast_chunks over any seekable reader `fh` of `size` bytes of blastout text (a file, compressed.BgzfReader)."""
+    chunks, start = [], 0
+    while start < size:
+        want = start + target_bytes
+        if want >= size:
+            chunks.append((start, size - start))
+            break
+        # row start at or after `want`
+        fh.seek(want - 1)
+        buf = fh.read(WINDOW)
+        nl = buf.find(b"\n")
+        while nl < 0 and len(buf) < size - want + 1:
+            more = fh.read(WINDOW)
+            if not more:
                 break
-            # row start at or after `want`
-            fh.seek(want - 1)
-            buf = fh.read(WINDOW)
+            buf += more
             nl = buf.find(b"\n")
-            while nl < 0 and len(buf) < size - want + 1:
-                more = fh.read(WINDOW)
-                if not more:
-                    break
-                buf += more
-                nl = buf.find(b"\n")
-            if nl < 0:
-                chunks.append((start, size - start))
+        if nl < 0:
+            chunks.append((start, size - start))
+            break
+        row0 = want - 1 + nl + 1          # absolute offset of a row start
+        # query of the row before row0
+        back = min(row0 - start, WINDOW)
+        fh.seek(row0 - back)
+        tail = fh.read(back)
+        prev_start = tail.rfind(b"\n", 0, len(tail) - 1) + 1
+        prev_row = tail[prev_start:]
+        tab = prev_row.find(b"\t")
+        carry = prev_row[:tab] if tab >= 0 else prev_row.rstrip(b"\n")
+        # first change of query at or after row0
+        fh.seek(row0)
+        pos_abs, cut = row0, -1
+        while pos_abs < size:
+            buf = fh.read(WINDOW)
+            if not buf:
                 break
-            row0 = want - 1 + nl + 1          # absolute offset of a row start
-            # query of the row before row0
-            back = min(row0 - start, WINDOW)
-            fh.seek(row0 - back)
-            tail = fh.read(back)
-            prev_start = tail.rfind(b"\n", 0, len(tail) - 1) + 1
-            prev_row = tail[prev_start:]
-            tab = prev_row.find(b"\t")
-            carry = prev_row[:tab] if tab >= 0 else prev_row.rstrip(b"\n")
-            # first change of query at or after row0
-            fh.seek(row0)
-            pos_abs, cut = row0, -1
-            while pos_abs < size:
-                buf = fh.read(WINDOW)
-                if not buf:
-                    break
+            last_nl = buf.rfind(b"\n")
+            if last_nl < 0:
+                more = fh.read(WINDOW)
+                while more and b"\n" not in more:
+                    buf += more
+                    more = fh.read(WINDOW)
+                buf += more
                 last_nl = buf.rfind(b"\n")
                 if last_nl < 0:
-                    more = fh.read(WINDOW)
-                    while more and b"\n" not in more:
-                        buf += more
-                        more = fh.read(WINDOW)
-                    buf += more
-                    last_nl = buf.rfind(b"\n")
-                    if last_nl < 0:
-                        break
-                body = buf[:last_nl + 1]
-                off, carry = _first_query_change(body, carry)
-                if off >= 0:
-                    cut = pos_abs + off
                     break
-                pos_abs += len(body)
-                fh.seek(pos_abs)
-            if cut < 0 or cut >= size:
-                chunks.append((start, size - start))
+            body = buf[:last_nl + 1]
+            off, carry = _first_query_change(body, carry)
+            if off >= 0:
+                cut = pos_abs + off
                 break
-            chunks.append((start, cut - start))
-            start = cut
+            pos_abs += len(body)
+            fh.seek(pos_abs)
+        if cut < 0 or cut >= size:
+            chunks.append((start, size - start))
+            break
+        chunks.append((start, cut - start))
+        start = cut
     return chunks
+
+
+def _text_cut(buf, target_bytes):
+    """Offset in `buf` (text from a row start) of the first query change at or after target_bytes, or -1 when the
+    complete rows of `buf` hold none."""
+    nl = buf.find(b"\n", max(target_bytes, 1) - 1)
+    if nl < 0:
+        return -1
+    row0 = nl + 1
+    prev_row = bytes(buf[buf.rfind(b"\n", 0, nl) + 1:nl])
+    tab = prev_row.find(b"\t")
+    off, _ = _first_query_change(bytes(buf[row0:]), prev_row[:tab] if tab >= 0 else prev_row)
+    return row0 + off if off >= 0 else -1
+
+
+def stream_text_chunks(path, target_bytes):
+    """The text of a generic gzip or bzip2 blastout, inflated as a stream (zlib and bz2 release the GIL), in pieces of
+    about target_bytes that start where the query name changes (the rule of scan_blast_chunks)."""
+    import bz2
+    import gzip
+    buf, eof = bytearray(), False
+    with (bz2.open if path.endswith(".bz2") else gzip.open)(path, "rb") as fh:
+        while True:
+            cut = _text_cut(buf, target_bytes) if len(buf) > target_bytes else -1
+            if cut > 0:
+                yield bytes(buf[:cut])
+                del buf[:cut]
+            elif eof:
+                if buf:
+                    yield bytes(buf)
+                return
+            else:
+                more = fh.read(max(WINDOW, target_bytes // 4))
+                buf += more
+                eof = not more
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -291,7 +330,7 @@ class ChunkScorer:
         self.parser = None
         self.known_taxa = set()
         self.n_systems = None
-        self.stats = dict(contigs=0, hits=0, ms_kernels=0.0, chunks=0)
+        self.stats = dict(contigs=0, hits=0, ms_kernels=0.0, chunks=0, inflated_members=0)
 
     def parse(self, text, genes=None):
         """The chunk's HitTable; with `genes` = (min_overlap, min_gene_length, min_scov) also its gene calls, as
@@ -318,6 +357,31 @@ class ChunkScorer:
             from . import genecaller
             calls = genecaller.call_genes(hits, *genes, device=self.device)[:5]
         return hits, calls
+
+    def parse_bgzf(self, buf, members, off, length, genes=None):
+        """`parse` of text bytes [off, off + length) of a BGZF blastout (bytes `buf`, member table `members`): the members
+        that hold them are inflated on the device and only those bytes are parsed.  A member that fails validation on the
+        device, or rows the device parser flags, send the chunk to the host (gzip raises its error on a bad member)."""
+        import gzip
+        from . import compressed
+        m0, m1 = compressed.member_range(members, off, length)
+        comp, sub = compressed.sub_table(buf, members, m0, m1)
+        own = (off - int(members[m0, compressed.OUT_OFF]), length) if m1 > m0 else (0, 0)
+        if not self.cpu_parse:
+            from . import gpu_parse
+            if self.parser is None:
+                self.parser = gpu_parse.BlastParser(self.device)
+            try:
+                hits = self.parser.parse_bgzf(comp, sub, own)
+            except gpu_parse.InflateError:
+                hits = None
+            if hits is not None:
+                self.stats["inflated_members"] += len(sub)
+                if genes is None:
+                    return hits
+                names = list(hits.block_names) if hits.block_names is not None else []
+                return hits, (names,) + self.parser.call_genes(*genes)
+        return self.parse(gzip.decompress(comp)[own[0]:own[0] + own[1]], genes)
 
     def score(self, names, hits, loci=None, details=None):
         """records of the contigs `names` given their parsed hits (possibly none); `loci`: the chunk's own LocusTable
@@ -369,28 +433,43 @@ class ChunkScorer:
             self.parser.close()
 
 
-def _worker(wid, device, path, tasks, results, shard_dir, args, tax, contig_lengths, loci_index, params_factory, engine_factory=None):
+def _worker(wid, device, path, members, tasks, results, shard_dir, args, tax, contig_lengths, loci_index, params_factory,
+            engine_factory=None):
+    """Tasks (chunk id, offset, length, chunk file): text bytes [offset, offset + length) of the blastout (a text file,
+    or the text of a BGZF file when `members` is its member table), or the whole of `chunk file` (a piece of a generic
+    gzip / bzip2 blastout the parent inflated; deleted once parsed)."""
+    import mmap
     try:
         scorer = ChunkScorer(device, args, tax, contig_lengths, loci_index, params_factory, cpu_parse=args.cpu_parse,
                              engine_factory=engine_factory)
+        genes = loci_index.thresholds if isinstance(loci_index, ChunkGenes) else None
         with open(path, "rb") as fh:
+            buf = mmap.mmap(fh.fileno(), 0, access=mmap.ACCESS_READ) if members is not None else None
             while True:
                 task = tasks.get()
                 if task is None:
                     break
-                cid, off, length = task
-                fh.seek(off)
-                text = fh.read(length)
+                cid, off, length, chunk_file = task
+                if chunk_file is not None:
+                    with open(chunk_file, "rb") as cf:
+                        text = cf.read()
+                    os.remove(chunk_file)
+                    parsed = scorer.parse(text, genes)
+                elif buf is not None:
+                    parsed = scorer.parse_bgzf(buf, members, off, length, genes)
+                else:
+                    fh.seek(off)
+                    parsed = scorer.parse(fh.read(length), genes)
                 prefix = os.path.join(shard_dir, "chunk{:06d}".format(cid))
                 loci = None
-                if isinstance(loci_index, ChunkGenes):
+                if genes is not None:
                     from . import genecaller
-                    hits, genes = scorer.parse(text, loci_index.thresholds)
-                    loci = parsers.LocusTable.from_blocks(*genes)
+                    hits, calls = parsed
+                    loci = parsers.LocusTable.from_blocks(*calls)
                     if loci_index.gff is not None:
-                        genecaller.write_gff(prefix + ".gff", *genes)
+                        genecaller.write_gff(prefix + ".gff", *calls)
                 else:
-                    hits = scorer.parse(text)
+                    hits = parsed
                 names = chunk_contigs(hits, contig_lengths)
                 records, scored = scorer.score(names, hits, loci,
                                                details=prefix + ".details.gz" if args.write_details else None)
@@ -405,6 +484,54 @@ def _worker(wid, device, path, tasks, results, shard_dir, args, tax, contig_leng
         results.put(("error", device, None, None, traceback.format_exc() or repr(exc)))
 
 
+class _TextFeeder:
+    """Parent-side reader of a generic gzip / bzip2 blastout: a thread inflates it as a stream, writes each piece
+    (stream_text_chunks) to a file in the shard directory and queues it as a task.  At most `slots` files exist at once;
+    the parent frees a slot when a worker reports the chunk."""
+
+    def __init__(self, path, chunk_bytes, shard_dir, tasks, n_workers):
+        import threading
+        self.n_chunks, self.error = None, None
+        self.slots = threading.Semaphore(2 * n_workers)
+        self._stop = threading.Event()
+        self._thread = threading.Thread(target=self._run, args=(path, chunk_bytes, shard_dir, tasks, n_workers),
+                                        daemon=True)
+
+    def start(self):   # after the workers are forked: a fork must not copy a thread mid-inflate
+        self._thread.start()
+
+    def _run(self, path, chunk_bytes, shard_dir, tasks, n_workers):
+        n = 0
+        try:
+            for cid, text in enumerate(stream_text_chunks(path, chunk_bytes)):
+                self.slots.acquire()
+                if self._stop.is_set():
+                    return
+                name = os.path.join(shard_dir, "text{:06d}".format(cid))
+                with open(name, "wb") as fh:
+                    fh.write(text)
+                tasks.put((cid, 0, len(text), name))
+                n += 1
+        except BaseException as exc:   # noqa: B902 -- re-raised in the parent (a corrupt file: gzip's / bz2's error)
+            self.error = exc
+        finally:
+            self.n_chunks = n
+            for _ in range(n_workers):
+                tasks.put(None)
+
+    def finish(self):
+        self._thread.join()
+        if self.error is not None:
+            raise self.error
+        return self.n_chunks
+
+    def stop(self):
+        self._stop.set()
+        self.slots.release()
+        if self._thread.is_alive():
+            self._thread.join()
+
+
 def run_streaming(args, tax, contig_lengths, loci, params_factory, devices, chunk_bytes, engine_factory=None):
     """The whole streamed run: returns (per-worker stats keyed by worker index, plus "rest"; number of chunks).  `loci`: a
     LocusTable, or a ChunkGenes (every chunk is scored against its own gene calls).  `devices`: CUDA device indices, one worker process each.  The
@@ -414,20 +541,36 @@ def run_streaming(args, tax, contig_lengths, loci, params_factory, devices, chun
     import shutil
     import tempfile
     from . import engine as _engine
+    from . import compressed
     loci_index = loci if isinstance(loci, ChunkGenes) else LociIndex(loci, contig_lengths)
-    chunks = scan_blast_chunks(args.blastout, chunk_bytes) if os.path.getsize(args.blastout) > 0 else []
+    fmt, members = compressed.classify(args.blastout)
+    chunks = None   # generic gzip / bzip2: cut while a thread inflates the stream (_TextFeeder)
+    if fmt == compressed.BGZF:   # chunks of the BGZF text, cut where the query changes; workers inflate on the device
+        import mmap
+        with open(args.blastout, "rb") as fh, mmap.mmap(fh.fileno(), 0, access=mmap.ACCESS_READ) as buf:
+            reader = compressed.BgzfReader(buf, members)
+            chunks = scan_text_chunks(reader, reader.size, chunk_bytes)
+    elif fmt == compressed.TEXT:
+        chunks = scan_blast_chunks(args.blastout, chunk_bytes) if os.path.getsize(args.blastout) > 0 else []
     shard_dir = tempfile.mkdtemp(prefix="wfl_shards_", dir=args.outdir)
     ctx = mp.get_context("spawn" if _engine.cuda_touched() else "fork")
     tasks, results = ctx.Queue(), ctx.Queue()
-    for cid, (off, length) in enumerate(chunks):
-        tasks.put((cid, off, length))
-    for _ in devices:
-        tasks.put(None)
-    procs = [ctx.Process(target=_worker, args=(w, d, args.blastout, tasks, results, shard_dir, args, tax, contig_lengths,
-                                               loci_index, params_factory, engine_factory), daemon=True)
+    feeder, n_chunks = None, None
+    if chunks is None:
+        feeder = _TextFeeder(args.blastout, chunk_bytes, shard_dir, tasks, len(devices))
+    else:
+        n_chunks = len(chunks)
+        for cid, (off, length) in enumerate(chunks):
+            tasks.put((cid, off, length, None))
+        for _ in devices:
+            tasks.put(None)
+    procs = [ctx.Process(target=_worker, args=(w, d, args.blastout, members, tasks, results, shard_dir, args, tax,
+                                               contig_lengths, loci_index, params_factory, engine_factory), daemon=True)
              for w, d in enumerate(devices)]
     for p in procs:
         p.start()
+    if feeder is not None:
+        feeder.start()
     prefixes, seen, stats, done = {}, set(), {}, 0
     try:
         import queue
@@ -445,6 +588,8 @@ def run_streaming(args, tax, contig_lengths, loci, params_factory, devices, chun
                 stats[a] = d
                 done += 1
                 continue
+            if feeder is not None:
+                feeder.slots.release()
             dup = seen.intersection(c)
             if dup:
                 die("blastout is not grouped by query sequence")   # UT:255-258
@@ -452,6 +597,8 @@ def run_streaming(args, tax, contig_lengths, loci, params_factory, devices, chun
             prefixes[a] = b
         for p in procs:
             p.join()
+        if feeder is not None:
+            n_chunks = feeder.finish()
         # contigs without a single hit: scored like the others (unclassified rows with their loci), in the parent's
         # process on the first device -- after the workers are gone
         rest = [nm for nm in contig_lengths if nm not in seen]
@@ -464,18 +611,20 @@ def run_streaming(args, tax, contig_lengths, loci, params_factory, devices, chun
                 records, _ = scorer.score(rest[k:k + step], empty)
                 prefix = os.path.join(shard_dir, "rest{:06d}".format(k // step))
                 write_shard(records, prefix)
-                prefixes[len(chunks) + k // step] = prefix
+                prefixes[n_chunks + k // step] = prefix
             stats["rest"] = dict(scorer.stats, device=devices[0])
             scorer.close()
         merge_shards([prefixes[k] for k in sorted(prefixes)], args.outdir, args.basename)
         if args.write_details:   # the contigs without hits ("rest") are never evaluated and have no rows (OS:959)
             writer.concat_details_shards(os.path.join(args.outdir, args.basename + ".details.tsv.gz"),
-                                         [prefixes[k] + ".details.gz" for k in range(len(chunks))])
+                                         [prefixes[k] + ".details.gz" for k in range(n_chunks)])
         if isinstance(loci_index, ChunkGenes) and loci_index.gff is not None:
-            concat_gff_shards([prefixes[k] + ".gff" for k in range(len(chunks))], loci_index.gff)
+            concat_gff_shards([prefixes[k] + ".gff" for k in range(n_chunks)], loci_index.gff)
     finally:
+        if feeder is not None:
+            feeder.stop()
         for p in procs:
             if p.is_alive():
                 p.terminate()
         shutil.rmtree(shard_dir, ignore_errors=True)
-    return stats, len(chunks)
+    return stats, n_chunks
