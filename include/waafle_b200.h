@@ -275,6 +275,35 @@ int64_t wfl_parser_call_genes(wfl_parser *p, double min_overlap, double min_gene
  * [n_genes] (strand: '+' / '-').  WFL_ERR_STATE before any gene call since the last wfl_parse_blast. */
 int  wfl_parser_genes_fetch(wfl_parser *p, int64_t *gene_off, int32_t *start, int32_t *end, int8_t *strand);
 
+/* ---- the scoring batch built from a parser's resident hit columns ----------------------------------------------------
+ * The wide wfl_batch of the parser's last wfl_parse_blast / wfl_parse_blast_resident, built in the engine's input
+ * buffers without the hit columns crossing PCIe.  Contig c takes parser rows [hit_src[c], hit_src[c] + hit_off[c+1] -
+ * hit_off[c]) (one blastout block); the taxon becomes slot_node[slot of the row's taxon] (the slots of
+ * wfl_parse_distinct kind 0); the annotation systems are re-ordered through sys_perm as wfl_parse_fetch does.  Without
+ * annotation systems (n_systems == 0) every contig's hits are ordered as Batch.sort_hits (waafle_b200/packing.py) orders
+ * them on the host, so the batch is byte for byte the one the host packer would upload.  Loci and offsets come from
+ * the host as in wfl_batch. */
+typedef struct {
+    int64_t n_contigs, n_hits, n_loci;
+    const int64_t *hit_off;        /* [n_contigs+1] host */
+    const int64_t *hit_src;        /* [n_contigs]  first parser row of contig c's block */
+    const int32_t *slot_node;      /* [2^20] distinct-taxon slot -> node index, -1 unused */
+    const int32_t *sys_perm;       /* [64] as wfl_parse_fetch; NULL when n_systems == 0 */
+    const int64_t *locus_off; const int32_t *locus_start, *locus_end; const int8_t *locus_strand;
+} wfl_parsed_batch;
+/* Leaves a resident batch that wfl_run_resident, wfl_download_results, wfl_pack_results and wfl_details_* use exactly
+ * like one from wfl_upload_batch.  The engine's stream waits for the parser's stream; the call returns when the batch is
+ * in place (*ms_kernels, NULL = skip: device time of the gather and sort kernels).  Errors, after which the engine has no
+ * batch: WFL_ERR_STATE when the parser's last parse flagged rows (or none was made) or params / taxonomy are missing;
+ * WFL_ERR_ARG when the parser is on another device, offsets do not span or are not monotone, a contig's row range lies
+ * outside the parser's rows, a hit's slot maps to -1 or to a node >= n_nodes, or sys_perm is NULL with n_systems > 0
+ * or given with n_systems == 0. */
+int  wfl_upload_parsed(wfl_engine *e, const wfl_parser *p, const wfl_parsed_batch *in, float *ms_kernels);
+/* Test hook: the hit columns of the resident wide batch to the host (each [n_hits], NULL = skip; sysmask only with
+ * n_systems > 0).  WFL_ERR_STATE without a resident wide batch. */
+int  wfl_debug_resident_batch(wfl_engine *e, int32_t *qstart, int32_t *qend, int32_t *taxon, double *score,
+                              double *scov, int8_t *strand, uint32_t *sysmask);
+
 /* ---- --write-details (waafle_orgscorer.py:766-812) -----------------------------------------------------------------
  * With the option "details" = <capacity> set (wfl_set_option) every run goes through the exact pipeline and records, per
  * contig and evaluated taxonomy level, every gene score of every clade (write_details :802-812 walks contig.gene_scores):

@@ -8,8 +8,9 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 SOURCES = ["wfl_fast.cu", "wfl_pipeline.cu", "wfl_compact.cu", "wfl_parse.cu", "wfl_genecall.cu", "wfl_details.cu", "wfl_inflate.cu",
-           "wfl_capi.cu"]
+           "wfl_resident_batch.cu", "wfl_capi.cu"]
 HEADERS = [os.path.join(HERE, "csrc", "wfl_device.cuh"), os.path.join(HERE, "csrc", "wfl_warp_common.cuh"),
+           os.path.join(HERE, "csrc", "wfl_warp_sort.cuh"),
            os.path.join(HERE, "csrc", "wfl_parser.cuh"), os.path.join(ROOT, "include", "waafle_b200.h")]
 LIB = os.path.join(HERE, "libwaafle_b200.so")
 

@@ -10,6 +10,7 @@
 #include <vector>
 
 #include "wfl_device.cuh"
+#include "wfl_parser.cuh"
 
 using namespace wfl;
 
@@ -52,6 +53,7 @@ struct wfl_engine {
     // device buffers (grow-only)
     Buf tx[4], anc, in[12], out[18], ctr, work, scratch, cm[5], dbg[4], plan_index, plan_data;
     Buf fb_list, fast_scratch, fast_wq, blob, status_tmp;
+    Buf rb_src, rb_lut, rb_perm, rb_red, rb_list, rb_scratch;   // wfl_upload_parsed: its inputs, reductions, sort scratch
     Buf det[6];                          // --write-details dump: contig, iteration, clade, locus, score, count
     int64_t det_cap = 0, det_used = 0;
     // --write-details text (wfl_details.cu): clade names of the taxonomy, state of the last wfl_details_prepare
@@ -867,7 +869,8 @@ int run_kernels(wfl_engine *e, bool streamed, wfl_results *out) {
     return WFL_ERR_CUDA;
 }
 
-int stage_inputs(wfl_engine *e, const HostBatch &in, bool copy_all) {
+// `host_hits` false: the hit columns are left to the caller (wfl_upload_parsed fills them on the device).
+int stage_inputs(wfl_engine *e, const HostBatch &in, bool copy_all, bool host_hits = true) {
     if (!e->have_params || !e->have_tax) {
         set_err(e, "set params and taxonomy before uploading a batch");
         return WFL_ERR_STATE;
@@ -933,7 +936,8 @@ int stage_inputs(wfl_engine *e, const HostBatch &in, bool copy_all) {
         }
     } else {
         for (int i = 0; i < in.ncol; ++i)
-            if (in.col[i] && nh) CU(cudaMemcpyAsync(dev_col(e, i), in.col[i], nh * in.esz[i], cudaMemcpyHostToDevice, os));
+            if (in.col[i] && nh && host_hits)
+                CU(cudaMemcpyAsync(dev_col(e, i), in.col[i], nh * in.esz[i], cudaMemcpyHostToDevice, os));
         if (nl) {
             CU(cudaMemcpyAsync(e->in[9].p, in.locus_start, nl * 4, cudaMemcpyHostToDevice, os));
             CU(cudaMemcpyAsync(e->in[10].p, in.locus_end, nl * 4, cudaMemcpyHostToDevice, os));
@@ -1100,6 +1104,140 @@ int details_rows(wfl_engine *e, int64_t s0, int64_t s1, char *text) {
     return WFL_OK;
 }
 
+// ---- the scoring batch from a parser's resident hit columns (wfl_resident_batch.cu) ----
+constexpr int PARSED_TAX_SLOTS = 1 << 20;   // the parser's distinct-taxon set (wfl_parse.cu)
+
+int upload_parsed(wfl_engine *e, const wfl_parser *p, const wfl_parsed_batch *in, float *ms_kernels) {
+    if (p->device != e->device) {
+        set_err(e, "the parser is on cuda:%d, the engine on cuda:%d", p->device, e->device);
+        return WFL_ERR_ARG;
+    }
+    if (!p->blast_ok) { set_err(e, "the parser holds no blastout parse without flagged rows"); return WFL_ERR_STATE; }
+    if (!e->have_params || !e->have_tax) { set_err(e, "set params and taxonomy before uploading a batch"); return WFL_ERR_STATE; }
+    const int S = e->P.p.n_systems;
+    HostBatch h;
+    h.n = in->n_contigs; h.nh = in->n_hits; h.nl = in->n_loci;
+    h.hit_off = in->hit_off; h.locus_off = in->locus_off;
+    h.locus_start = in->locus_start; h.locus_end = in->locus_end; h.locus_strand = in->locus_strand;
+    // the sources of the wide columns: qstart qend taxon-slot score scov strand on the device, the system map on the host
+    const void *c[7] = {p->col[0].p, p->col[1].p, p->col[5].p, p->col[2].p, p->col[3].p, p->col[4].p,
+                        S > 0 ? in->sys_perm : nullptr};
+    const int z[7] = {4, 4, 4, 8, 8, 1, 4};
+    for (int i = 0; i < 7; ++i) { h.col[i] = c[i]; h.esz[i] = z[i]; }
+    h.ncol = 7;
+    if ((S > 0) != (in->sys_perm != nullptr)) {
+        set_err(e, "sys_perm must be given exactly when n_systems > 0");
+        return WFL_ERR_ARG;
+    }
+    int rc = check_host_batch(e, h);
+    if (rc) return rc;
+    if (h.nh && (!in->hit_src || !in->slot_node)) { set_err(e, "null array in batch"); return WFL_ERR_ARG; }
+    for (int64_t k = 0; k < h.n; ++k) {
+        const int64_t cnt = h.hit_off[k + 1] - h.hit_off[k];
+        if (cnt && (in->hit_src[k] < 0 || in->hit_src[k] > p->n_rows - cnt)) {
+            set_err(e, "contig %lld: rows [%lld, %lld) outside the parser's %lld rows", (long long)k,
+                    (long long)in->hit_src[k], (long long)(in->hit_src[k] + cnt), (long long)p->n_rows);
+            return WFL_ERR_ARG;
+        }
+    }
+    for (int b = 0; S > 0 && b < 64; ++b)
+        if (in->sys_perm[b] < -1 || in->sys_perm[b] >= 32) { set_err(e, "sys_perm[%d] out of range", b); return WFL_ERR_ARG; }
+    if ((rc = stage_inputs(e, h, true, false))) return rc;
+    e->have_batch = false;   // until the hit columns are in place
+    const int64_t n = h.n, nh = h.nh;
+    // sort plan (host knows every contig's size): contigs whose keys exceed a first-launch slice go to a second launch
+    const bool sort = S == 0 && nh > 0;
+    const long long slice1 = 32 << 10, warps1 = std::min<long long>((long long)e->sm_count * 64, (n + 7) & ~7ll);
+    long long slice2 = 0;
+    std::vector<int> big;
+    for (int64_t k = 0; sort && k < n; ++k) {
+        long long np2 = 1;
+        while (np2 < h.hit_off[k + 1] - h.hit_off[k]) np2 <<= 1;
+        if (16 * np2 > slice1) { big.push_back((int)k); slice2 = std::max(slice2, 16 * np2); }
+    }
+    const long long warps2 = big.empty() ? 0 : (std::max<long long>(1, std::min<long long>((long long)big.size(), (1ll << 30) / slice2)) + 7) & ~7ll;
+    int64_t *d_src;
+    int32_t *d_lut, *d_perm, *d_list = nullptr;
+    unsigned long long *d_red;
+    char *scratch = nullptr;
+    if ((rc = outbuf(e, e->rb_src, (size_t)std::max<int64_t>(n, 1), &d_src)) ||
+        (rc = outbuf(e, e->rb_lut, PARSED_TAX_SLOTS, &d_lut)) || (rc = outbuf(e, e->rb_perm, 64, &d_perm)) ||
+        (rc = outbuf(e, e->rb_red, 3, &d_red)) ||
+        (sort && (rc = outbuf(e, e->rb_scratch, (size_t)std::max(slice1 * warps1, slice2 * warps2), &scratch))) ||
+        (!big.empty() && (rc = outbuf(e, e->rb_list, big.size(), &d_list))))
+        return rc;
+    if (n && in->hit_src) CU(cudaMemcpyAsync(d_src, in->hit_src, (size_t)n * 8, cudaMemcpyHostToDevice, e->stream));
+    if (in->slot_node) CU(cudaMemcpyAsync(d_lut, in->slot_node, (size_t)PARSED_TAX_SLOTS * 4, cudaMemcpyHostToDevice, e->stream));
+    if (S > 0) CU(cudaMemcpyAsync(d_perm, in->sys_perm, 64 * 4, cudaMemcpyHostToDevice, e->stream));
+    if (!big.empty()) CU(cudaMemcpyAsync(d_list, big.data(), big.size() * 4, cudaMemcpyHostToDevice, e->stream));
+    CU(cudaMemsetAsync(d_red, 0, 3 * sizeof(unsigned long long), e->stream));
+    // the parse (and anything else queued on the parser's stream) comes first
+    CU(cudaEventRecord(e->ev_join, p->stream));
+    CU(cudaStreamWaitEvent(e->stream, e->ev_join, 0));
+    CU(cudaEventRecord(e->ev[1], e->stream));
+    ResBatchArgs a{};
+    a.qstart = static_cast<const int32_t *>(p->col[0].p); a.qend = static_cast<const int32_t *>(p->col[1].p);
+    a.score = static_cast<const double *>(p->col[2].p); a.scov = static_cast<const double *>(p->col[3].p);
+    a.strand = static_cast<const int8_t *>(p->col[4].p); a.tcode = static_cast<const int32_t *>(p->col[5].p);
+    a.rawmask = static_cast<const unsigned long long *>(p->col[6].p);
+    a.hit_off = e->b.hit_off; a.hit_src = d_src;
+    a.n = n; a.nh = nh;
+    a.slot_node = d_lut; a.n_slots = PARSED_TAX_SLOTS; a.n_nodes = e->tax.n_nodes;
+    a.sys_perm = S > 0 ? d_perm : nullptr;
+    a.o_qstart = static_cast<int32_t *>(dev_col(e, 0)); a.o_qend = static_cast<int32_t *>(dev_col(e, 1));
+    a.o_taxon = static_cast<int32_t *>(dev_col(e, 2)); a.o_score = static_cast<double *>(dev_col(e, 3));
+    a.o_scov = static_cast<double *>(dev_col(e, 4)); a.o_strand = static_cast<int8_t *>(dev_col(e, 5));
+    a.o_sysmask = S > 0 ? static_cast<uint32_t *>(dev_col(e, 6)) : nullptr;
+    a.red = d_red;
+    unsigned long long red[3] = {0, 0, 0};
+    if (nh) {
+        launch_resident_gather(a, e->sm_count, e->stream);
+        CU(cudaGetLastError());
+        CU(cudaEventRecord(e->ev[3], e->stream));
+        CU(cudaMemcpyAsync(red, d_red, sizeof red, cudaMemcpyDeviceToHost, e->stream));
+    }
+    CU(cudaStreamSynchronize(e->stream));
+    if (red[0]) {
+        set_err(e, "%llu hits carry a taxon slot that maps to no taxonomy node", red[0]);
+        return WFL_ERR_ARG;
+    }
+    if (sort) {
+        // Batch.sort_hits' choice of key
+        int bits_c = 1, bits_t = 1;
+        while (bits_c < 63 && (1ll << bits_c) <= n - 1) ++bits_c;
+        while (bits_t < 63 && (1ull << bits_t) <= red[2]) ++bits_t;
+        const int bits_s = 63 - bits_c - bits_t;
+        double smax;
+        memcpy(&smax, &red[1], 8);
+        a.quantised = bits_s >= 20 && smax > 0.0;
+        a.bits_s = bits_s;
+        a.smax = smax;
+        a.scratch = scratch;
+        a.slice = slice1;
+        CU(cudaEventRecord(e->ev[4], e->stream));
+        launch_resident_sort(a, warps1, e->stream);
+        CU(cudaGetLastError());
+        if (!big.empty()) {
+            a.list = d_list;
+            a.n_list = (long long)big.size();
+            a.slice = slice2;
+            launch_resident_sort(a, warps2, e->stream);
+            CU(cudaGetLastError());
+        }
+    }
+    CU(cudaEventRecord(e->ev[2], e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    if (ms_kernels) {   // the gather, plus the sort when there is one (not the host's wait in between)
+        float t = 0.f;
+        *ms_kernels = 0.f;
+        if (nh) CU(cudaEventElapsedTime(ms_kernels, e->ev[1], e->ev[3]));
+        if (sort) CU(cudaEventElapsedTime(&t, e->ev[4], e->ev[2]));
+        *ms_kernels += t;
+    }
+    e->have_batch = true;
+    return WFL_OK;
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------
@@ -1189,6 +1327,7 @@ void wfl_destroy(wfl_engine *e) {
                    &e->dt_scratch, &e->dt_defer[0], &e->dt_defer[1], &e->dt_ctr, &e->dt_text})
         fr(*b);
     fr(e->fb_list); fr(e->fast_scratch); fr(e->fast_wq); fr(e->blob); fr(e->status_tmp);
+    for (Buf *b : {&e->rb_src, &e->rb_lut, &e->rb_perm, &e->rb_red, &e->rb_list, &e->rb_scratch}) fr(*b);
     for (int q = 0; q < 2; ++q) { fr(e->pipe_pool[q]); fr(e->pipe_lists[q]); fr(e->pipe_cnt[q]); fr(e->pipe_wq[q]); }
     fr(e->pipe_ctg);
     for (int q = 0; q < 2; ++q) { fr(e->k2_desc[q]); fr(e->k2_order[q]); fr(e->k2_keys[q]); fr(e->k2_meta[q]); }
@@ -1291,6 +1430,31 @@ int wfl_upload_packed(wfl_engine *e, const wfl_packed_batch *in) {
     if (!e || !in) return WFL_ERR_ARG;
     CU(cudaSetDevice(e->device));
     return stage_inputs(e, host_batch(in, e->P.p.n_systems), true);
+}
+
+int wfl_upload_parsed(wfl_engine *e, const wfl_parser *p, const wfl_parsed_batch *in, float *ms_kernels) {
+    if (!e || !p || !in) return WFL_ERR_ARG;
+    CU(cudaSetDevice(e->device));
+    e->have_batch = e->have_results = false;
+    const int rc = upload_parsed(e, p, in, ms_kernels);
+    if (rc) {
+        cudaStreamSynchronize(e->stream);   // nothing of ours reads the caller's arrays after an error
+        e->have_batch = e->have_results = false;
+    }
+    return rc;
+}
+
+int wfl_debug_resident_batch(wfl_engine *e, int32_t *qstart, int32_t *qend, int32_t *taxon, double *score, double *scov,
+                             int8_t *strand, uint32_t *sysmask) {
+    if (!e) return WFL_ERR_ARG;
+    CU(cudaSetDevice(e->device));
+    if (!e->have_batch || e->packed) { set_err(e, "no resident batch in the wide format"); return WFL_ERR_STATE; }
+    void *dst[7] = {qstart, qend, taxon, score, scov, strand, e->S > 0 ? sysmask : nullptr};
+    const size_t esz[7] = {4, 4, 4, 8, 8, 1, 4};
+    for (int i = 0; i < 7; ++i)
+        if (dst[i] && e->nh) CU(cudaMemcpyAsync(dst[i], dev_col(e, i), (size_t)e->nh * esz[i], cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    return WFL_OK;
 }
 
 int wfl_run_resident(wfl_engine *e) {

@@ -9,7 +9,7 @@
 // The same code counts (length pass, text == null) and writes (write pass).
 #include <algorithm>
 
-#include "wfl_warp_common.cuh"
+#include "wfl_warp_sort.cuh"
 
 namespace wfl {
 namespace {
@@ -73,33 +73,6 @@ struct Sink {
         while (k) put(t[--k]);
     }
 };
-
-// 128-bit keys (hi, lo), ascending; a warp sorts n (a power of two) of them in place (bitonic network)
-__device__ __forceinline__ bool key_less(const ulonglong2 &a, const ulonglong2 &b) {
-    return a.x < b.x || (a.x == b.x && a.y < b.y);
-}
-__device__ __noinline__ void warp_sort(ulonglong2 *v, int n) {
-#pragma unroll 1
-    for (int k = 2; k <= n; k <<= 1)
-#pragma unroll 1
-        for (int j = k >> 1; j > 0; j >>= 1) {
-#pragma unroll 1
-            for (int i = lane_id(); i < n; i += 32) {
-                const int ij = i ^ j;
-                if (ij > i) {
-                    const ulonglong2 a = v[i], b = v[ij];
-                    if (((i & k) == 0) == key_less(b, a)) { v[i] = b; v[ij] = a; }
-                }
-            }
-            __syncwarp();
-        }
-}
-
-__device__ __forceinline__ int pow2_at_least(int n) {
-    int p = 1;
-    while (p < n) p <<= 1;
-    return p;
-}
 
 // scratch bytes of one segment: retained loci, row heads, the two key arrays
 __device__ __forceinline__ long long seg_need(int G, int len, int M) {

@@ -251,6 +251,37 @@ void launch_details_segments(const DetTextArgs &a, cudaStream_t s);
 void launch_details_rows(const DetTextArgs &a, long long warps, cudaStream_t s);
 void launch_format3(const double *x, long long n, char *text, int *len, unsigned int *err, cudaStream_t s);
 
+// ---- the wide scoring batch built from a parser's resident hit columns (wfl_resident_batch.cu) ------------------
+struct ResBatchArgs {
+    // the parser's columns, one entry per parsed row
+    const int32_t *qstart, *qend, *tcode;
+    const double *score, *scov;
+    const int8_t *strand;
+    const unsigned long long *rawmask;
+    // the batch: contig c takes rows [hit_src[c], hit_src[c] + hit_off[c + 1] - hit_off[c])
+    const int64_t *hit_off, *hit_src;
+    long long n, nh;
+    const int32_t *slot_node;      // distinct-taxon slot -> node index
+    int n_slots, n_nodes;
+    const int32_t *sys_perm;       // [64] raw system bit -> bit in the sorted system list; null: no systems, hits sorted
+    // outputs: the engine's wide input columns
+    int32_t *o_qstart, *o_qend, *o_taxon;
+    double *o_score, *o_scov;
+    int8_t *o_strand;
+    uint32_t *o_sysmask;
+    unsigned long long *red;       // [0] hits with an unusable slot, [1] bits of the largest finite score > 0, [2] largest node
+    // sort (Batch.sort_hits): quantised (taxon << bits_s | q, row) or lexsort (taxon, -score, row) keys
+    bool quantised;
+    int bits_s;
+    double smax;
+    const int *list;               // contigs of the second launch, or null: every contig whose keys fit `slice`
+    long long n_list;
+    char *scratch;                 // `slice` bytes per warp
+    long long slice;
+};
+void launch_resident_gather(const ResBatchArgs &a, int sm_count, cudaStream_t s);   // checks, reductions; copies if unsorted
+void launch_resident_sort(const ResBatchArgs &a, long long warps, cudaStream_t s);
+
 // Compaction (K10): CSR of melded members in contig order + contig indices grouped by call.
 struct CompactArgs {
     int64_t n;

@@ -29,7 +29,7 @@ EXPORTS = ["wfl_abi_version", "wfl_device_count", "wfl_create", "wfl_destroy", "
            "wfl_host_free", "wfl_parser_create", "wfl_parser_destroy", "wfl_parser_last_error", "wfl_parse_blast",
            "wfl_parse_blast_resident", "wfl_parser_text", "wfl_inflate_bgzf", "wfl_parse_distinct", "wfl_parse_fetch", "wfl_parser_times", "wfl_call_genes", "wfl_download_details", "wfl_parse_gff", "wfl_parse_gff_fetch",
            "wfl_parser_call_genes", "wfl_parser_genes_fetch", "wfl_set_clade_names", "wfl_details_prepare",
-           "wfl_details_text", "wfl_debug_format_scores"]
+           "wfl_details_text", "wfl_debug_format_scores", "wfl_upload_parsed", "wfl_debug_resident_batch"]
 ABI_VERSION = 2
 _CUDA_TOUCHED = False   # this process has initialised CUDA through the library (a fork could not use it any more)
 
@@ -61,6 +61,13 @@ class CPackedBatch(ctypes.Structure):
                 ("hit_qstart16", c_u16p), ("hit_qend16", c_u16p), ("hit_tax16", c_u16p),
                 ("hit_score", c_f64p), ("hit_sysmask8", c_u8p),
                 ("locus_start", c_i32p), ("locus_end", c_i32p), ("locus_strand", c_i8p)]
+
+
+class CParsedBatch(ctypes.Structure):
+    """`wfl_parsed_batch` (the scoring batch built from a parser's device columns)."""
+    _fields_ = [("n_contigs", ctypes.c_int64), ("n_hits", ctypes.c_int64), ("n_loci", ctypes.c_int64),
+                ("hit_off", c_i64p), ("hit_src", c_i64p), ("slot_node", c_i32p), ("sys_perm", c_i32p),
+                ("locus_off", c_i64p), ("locus_start", c_i32p), ("locus_end", c_i32p), ("locus_strand", c_i8p)]
 
 
 class CResults(ctypes.Structure):
@@ -138,6 +145,9 @@ def load_library(path=None):
     lib.wfl_details_text.restype = ctypes.c_int64
     lib.wfl_debug_format_scores.argtypes = [ctypes.c_void_p, c_f64p, ctypes.c_int64, ctypes.c_void_p, c_i32p]
     lib.wfl_debug_format_scores.restype = ctypes.c_int64
+    lib.wfl_upload_parsed.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.POINTER(CParsedBatch),
+                                      ctypes.POINTER(ctypes.c_float)]
+    lib.wfl_debug_resident_batch.argtypes = [ctypes.c_void_p, c_i32p, c_i32p, c_i32p, c_f64p, c_f64p, c_i8p, c_u32p]
     lib.wfl_host_alloc.argtypes = [ctypes.c_size_t, ctypes.POINTER(ctypes.c_void_p)]
     lib.wfl_host_free.argtypes = [ctypes.c_void_p]
     lib.wfl_host_free.restype = None
@@ -214,6 +224,7 @@ class Engine:
         self.n_systems = 0
         self._clade_names = None        # names of the taxonomy's nodes, uploaded by the first details_text after set_taxonomy
         self.details_times = {}
+        self.resident_times = {}        # ms_kernels of the last upload_parsed
         if params is not None:
             self.set_params(params)
         if taxonomy is not None:
@@ -342,7 +353,12 @@ class Engine:
         return r
 
     def score_batch(self, batch):
-        """Host arrays in, host arrays out (H2D + kernels + D2H inside the call)."""
+        """Host arrays in, host arrays out (H2D + kernels + D2H inside the call).  A packing.ResidentBatch has its hit
+        columns built on the device from its parser's columns instead (upload_parsed, run_resident, download)."""
+        if hasattr(batch, "hit_src"):
+            self.upload_parsed(batch)
+            self.run_resident()
+            return self.download()
         cb, n, nh, nl, packed = self._cbatch(batch)
         call = self._lib.wfl_score_packed if packed else self._lib.wfl_score_batch
         cap = max(4 * n, 1024)
@@ -361,6 +377,45 @@ class Engine:
         call = self._lib.wfl_upload_packed if packed else self._lib.wfl_upload_batch
         self._check(call(self._h, ctypes.byref(cb)))
         self._resident = (n, nl)
+
+    def upload_parsed(self, batch):
+        """Build the resident wide batch of a packing.ResidentBatch on the device (wfl_upload_parsed) from the columns
+        its GPU parse left there; raises EngineError when that parse is no longer live (the parser was closed or has
+        parsed again since)."""
+        res = batch.resident
+        if res is None or not res.live:
+            raise EngineError("the batch's GPU parse is no longer live (its parser was closed or parsed again)")
+        k = dict(hit_off=_as(batch.hit_off, np.int64), hit_src=_as(batch.hit_src, np.int64),
+                 slot_node=_as(batch.slot_node, np.int32), locus_off=_as(batch.locus_off, np.int64),
+                 locus_start=_as(batch.locus_start, np.int32), locus_end=_as(batch.locus_end, np.int32),
+                 locus_strand=_as(batch.locus_strand, np.int8))
+        n, nl = len(k["hit_off"]) - 1, len(k["locus_start"])
+        pb = CParsedBatch(n_contigs=n, n_hits=int(k["hit_off"][-1]), n_loci=nl)
+        ftypes = dict(CParsedBatch._fields_)
+        for name, arr in k.items():
+            setattr(pb, name, _ptr(arr, ftypes[name]._type_))
+        if res.sys_perm is not None:
+            k["sys_perm"] = _as(res.sys_perm, np.int32)
+            pb.sys_perm = _ptr(k["sys_perm"], ctypes.c_int32)
+        self._keep = k
+        ms = ctypes.c_float()
+        self._check(self._lib.wfl_upload_parsed(self._h, res.parser._h, ctypes.byref(pb), ctypes.byref(ms)))
+        self.resident_times = dict(ms_kernels=ms.value)
+        self._resident = (n, nl)
+
+    def debug_resident_batch(self):
+        """The hit columns of the resident wide batch (test hook), as Batch.arrays() names them."""
+        nh = int(self._keep["hit_off"][-1]) if "hit_off" in self._keep else 0
+        out = dict(hit_qstart=np.empty(nh, np.int32), hit_qend=np.empty(nh, np.int32), hit_taxon=np.empty(nh, np.int32),
+                   hit_score=np.empty(nh, np.float64), hit_scov=np.empty(nh, np.float64), hit_strand=np.empty(nh, np.int8))
+        if self.n_systems > 0:
+            out["hit_sysmask"] = np.empty(nh, np.uint32)
+        self._check(self._lib.wfl_debug_resident_batch(
+            self._h, *[_ptr(out[k], t) for k, t in (("hit_qstart", ctypes.c_int32), ("hit_qend", ctypes.c_int32),
+                                                    ("hit_taxon", ctypes.c_int32), ("hit_score", ctypes.c_double),
+                                                    ("hit_scov", ctypes.c_double), ("hit_strand", ctypes.c_int8))],
+            _ptr(out["hit_sysmask"], ctypes.c_uint32) if "hit_sysmask" in out else None))
+        return out
 
     def run_resident(self):
         self._check(self._lib.wfl_run_resident(self._h))

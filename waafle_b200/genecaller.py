@@ -96,8 +96,9 @@ def main(argv=None):
     if args.gff is None:
         name = os.path.split(args.blastout)[1].split(".")[0]   # utils.path2name / name2path (:201-203)
         args.gff = os.path.join(".", name + ".gff")
-    _, genes = parsers.read_blast_hits_and_genes(args.blastout, args.min_overlap, args.min_gene_length, args.min_scov,
-                                                 device=args.device, cpu_parse=args.cpu_parse)
+    hits, genes = parsers.read_blast_hits_and_genes(args.blastout, args.min_overlap, args.min_gene_length, args.min_scov,
+                                                    device=args.device, cpu_parse=args.cpu_parse)
+    parsers.close_resident(hits)
     write_gff(args.gff, *genes)
     say("Finished successfully.")
 

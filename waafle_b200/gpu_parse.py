@@ -74,8 +74,30 @@ class _TextNames:
         return self._text[o:o + int(self._len[int(i)])].decode()
 
 
+class ResidentParse:
+    """The device columns a HitTable came from: parse number `generation` of `parser`.  `taxon_slots[k]`: the slot of the
+    HitTable's taxon_names[k] in the parser's distinct-taxon set; `sys_perm`: the system map of wfl_parse_fetch (None
+    without annotation systems).  packing.pack_resident builds the scoring batch from these columns on the device."""
+
+    def __init__(self, parser, generation, taxon_slots, sys_perm):
+        self.parser, self.generation = parser, generation
+        self.taxon_slots, self.sys_perm = taxon_slots, sys_perm
+
+    @property
+    def live(self):
+        """The parser is open and has not parsed anything since."""
+        return self.parser.is_open and self.parser.generation == self.generation
+
+
+def live_resident(hits):
+    """The ResidentParse of a HitTable whose parser still holds its columns, else None."""
+    r = getattr(hits, "resident", None)
+    return r if r is not None and r.live else None
+
+
 class BlastParser:
-    """One parser handle on one GPU."""
+    """One parser handle on one GPU.  `generation` counts the parses made with it: the device columns belong to the last
+    one only."""
 
     def __init__(self, device=0):
         self._lib = _lib()
@@ -85,7 +107,13 @@ class BlastParser:
         if rc != 0 or not h:
             raise EngineError("wfl_parser_create(device={}) failed with {}: no usable CUDA device".format(device, rc))
         self._h = h
+        self.device = int(device)
+        self.generation = 0
         self.times = {}
+
+    @property
+    def is_open(self):
+        return bool(getattr(self, "_h", None))
 
     def close(self):
         if getattr(self, "_h", None):
@@ -110,6 +138,7 @@ class BlastParser:
         flagged, first = ctypes.c_int32(), ctypes.c_int64()
         if len(text.strip()) == 0:   # an empty parse on the device too, so that call_genes sees no blocks
             text = b""
+        self.generation += 1
         n = self._lib.wfl_parse_blast(self._h, text, len(text), ctypes.byref(flagged), ctypes.byref(first))
         return self._collect(text, n, flagged)
 
@@ -144,6 +173,7 @@ class BlastParser:
         if len(text.strip()) == 0:
             off, n = 0, 0
         flagged, first = ctypes.c_int32(), ctypes.c_int64()
+        self.generation += 1
         rows = self._lib.wfl_parse_blast_resident(self._h, off, n, ctypes.byref(flagged), ctypes.byref(first))
         hits = self._collect(text if n else b"", rows, flagged)
         if hits is not None:
@@ -158,7 +188,9 @@ class BlastParser:
             return None
         if len(text) == 0:
             self.times = dict(ms_h2d=0.0, ms_kernels=0.0, ms_d2h=0.0, rows=0, bytes=0)
-            return parsers.hits_from_columns(*([[]] * 10))
+            hits = parsers.hits_from_columns(*([[]] * 10))
+            hits.resident = ResidentParse(self, self.generation, np.zeros(0, np.int64), None)
+            return hits
         n = int(n)
         # ---- the distinct names: taxa (2^20 slots) and annotation systems (64 slots) ----
         vp = lambda a: a.ctypes.data_as(ctypes.c_void_p)
@@ -193,11 +225,13 @@ class BlastParser:
         starts = np.flatnonzero(cols["newblock"]).astype(np.int64)
         block_names = [text[int(o):int(o) + int(l)].decode() for o, l in zip(cols["q_off"][starts], cols["q_len"][starts])]
         names = _TextNames(text, cols["ss_off"], cols["ss_len"])
-        return parsers.HitTable(
+        hits = parsers.HitTable(
             qseqid=None, qstart=cols["qstart"], qend=cols["qend"], taxon=None, score=cols["score"],
             scov_modified=cols["scov"], strand=cols["strand"], sseqid_id=None, sseqid_names=names,
             sseqid_annotations=parsers._LazyAnnotations(names), systems=systems, sysmask=cols["sysmask"],
             taxon_codes=tlut[cols["tcode"]], taxon_names=taxon_names, block_starts=starts, block_names=block_names)
+        hits.resident = ResidentParse(self, self.generation, tslots, perm if systems else None)
+        return hits
 
     def call_genes(self, min_overlap, min_gene_length, min_scov):
         """waafle_genecaller over the hit columns of the last `parse` (still on the device: no hit data is shipped again).
@@ -224,6 +258,7 @@ class BlastParser:
         if len(text.strip()) == 0:
             return parsers.LocusTable([], [], [], [])
         flagged, first = ctypes.c_int32(), ctypes.c_int64()
+        self.generation += 1
         n = self._lib.wfl_parse_gff(self._h, text, len(text), ctypes.byref(flagged), ctypes.byref(first))
         self._check(n)
         if flagged.value:

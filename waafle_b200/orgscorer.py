@@ -13,7 +13,7 @@ import functools
 import os
 import sys
 
-from . import packing, parsers, taxonomy, writer
+from . import gpu_parse, packing, parsers, taxonomy, writer
 from .engine import Engine
 from .params import OrgscorerParams
 from .utils import die, read_contig_lengths, say
@@ -175,7 +175,9 @@ def analyze(args, tax, contig_lengths, loci, hits=None):
     if hits.sysmask is None:
         die("more than 32 annotation systems in the subject headers")
     tax.build(hits.distinct_taxa())
-    batch = packing.pack(contig_lengths, loci, hits, tax)
+    # hits parsed on the GPU: the batch's hit columns are built there from the parser's columns
+    pack = packing.pack_resident if gpu_parse.live_resident(hits) is not None else packing.pack
+    batch = pack(contig_lengths, loci, hits, tax)
     params = OrgscorerParams.from_args(args, n_systems=len(hits.systems))
     engine = Engine(args.device, params, tax)
     if args.exact_scores:
@@ -195,6 +197,7 @@ def analyze(args, tax, contig_lengths, loci, hits=None):
         writer.write_details_file(os.path.join(args.outdir, args.basename + ".details.tsv.gz"),
                                   engine.details_text(details_order(batch, hits, contig_lengths), batch.contig_names))
     engine.close()
+    parsers.close_resident(hits)
     records = writer.build_records(batch, loci, hits, tax, res)
     writer.write_main_output_files(records, args.outdir, args.basename)
     say("Finished successfully.")

@@ -181,8 +181,20 @@ def _group(names, index, what, codes=None, code_names=None):
     return cid
 
 
-def pack(contig_lengths, loci, hits, taxonomy):
-    """Pack parsed inputs. `taxonomy` must already be built with the hit taxa as extra names."""
+def block_rows(hit_off, hit_src):
+    """Row of every packed hit in the HitTable when contig c holds rows [hit_src[c], hit_src[c] + its hit count)."""
+    counts = np.diff(hit_off)
+    n_hits = int(hit_off[-1])
+    return np.repeat(np.asarray(hit_src, np.int64) - hit_off[:-1], counts) + np.arange(n_hits, dtype=np.int64)
+
+
+def map_contigs(contig_lengths, loci, hits):
+    """Where the contigs of `pack` find their loci and hits: (names, locus_off, locus_row, hit_off, hit_src, hit_contig).
+    Contigs in FASTA order; unknown contigs are warned about and dropped (OS:921-923); a blastout that is not grouped
+    by query dies (UT:255-258).  Loci: locus_row[locus_off[c]:locus_off[c + 1]] are contig c's rows of `loci`.  Hits,
+    for a HitTable with block_starts (every contig is one block of rows): hit_src[c] = first row of contig c's block
+    (0 without hits), hit_contig = None; otherwise hit_src = None and hit_contig = the contig of every row (-1:
+    unknown)."""
     names = list(contig_lengths)
     index = {n: i for i, n in enumerate(names)}
     n = len(names)
@@ -193,28 +205,43 @@ def pack(contig_lengths, loci, hits, taxonomy):
     locus_off = np.zeros(n + 1, dtype=np.int64)
     np.cumsum(np.bincount(lc[lrow], minlength=n), out=locus_off[1:])
 
+    hit_off = np.zeros(n + 1, dtype=np.int64)
     if getattr(hits, "block_starts", None) is not None and len(hits):
         # run-length coded query names (GPU parser): one lookup per block, no per-row objects
         bcid = np.fromiter((index.get(nm, -1) for nm in hits.block_names), dtype=np.int64, count=len(hits.block_names))
         for nm in np.array(hits.block_names, dtype=object)[bcid < 0]:
             say("  Unknown contig in <{}> file".format("blastout"), nm)
-        known = bcid[bcid >= 0]
-        if len(np.unique(known)) != len(known):   # the reference assumes the blastout is grouped by query (UT:255-258)
+        known = bcid >= 0
+        if len(np.unique(bcid[known])) != int(known.sum()):   # the reference assumes the blastout is grouped by query (UT:255-258)
             die("blastout is not grouped by query sequence")
-        hc = np.repeat(bcid, np.diff(np.r_[hits.block_starts, len(hits)]))
+        starts = np.asarray(hits.block_starts, dtype=np.int64)
+        lens = np.diff(np.r_[starts, len(hits)])
+        counts = np.zeros(n, dtype=np.int64)
+        counts[bcid[known]] = lens[known]
+        np.cumsum(counts, out=hit_off[1:])
+        hit_src = np.zeros(n, dtype=np.int64)
+        hit_src[bcid[known]] = starts[known]
+        return names, locus_off, lrow, hit_off, hit_src, None
+    hc = _group(hits.qseqid, index, "blastout", getattr(hits, "qseqid_codes", None), getattr(hits, "qseqid_names", None))
+    if len(hc):
+        # the reference assumes the blastout is grouped by query (UT:255-258)
+        starts = np.r_[True, hits.qseqid[1:] != hits.qseqid[:-1]]
+        blocks = hc[starts]
+        blocks = blocks[blocks >= 0]
+        if len(np.unique(blocks)) != len(blocks):
+            die("blastout is not grouped by query sequence")
+    np.cumsum(np.bincount(hc[hc >= 0], minlength=n), out=hit_off[1:])
+    return names, locus_off, lrow, hit_off, None, hc
+
+
+def pack(contig_lengths, loci, hits, taxonomy):
+    """Pack parsed inputs. `taxonomy` must already be built with the hit taxa as extra names."""
+    names, locus_off, lrow, hit_off, hit_src, hc = map_contigs(contig_lengths, loci, hits)
+    if hc is None:
+        hrow = block_rows(hit_off, hit_src)
     else:
-        hc = _group(hits.qseqid, index, "blastout", getattr(hits, "qseqid_codes", None), getattr(hits, "qseqid_names", None))
-        if len(hc):
-            # the reference assumes the blastout is grouped by query (UT:255-258)
-            starts = np.r_[True, hits.qseqid[1:] != hits.qseqid[:-1]]
-            blocks = hc[starts]
-            blocks = blocks[blocks >= 0]
-            if len(np.unique(blocks)) != len(blocks):
-                die("blastout is not grouped by query sequence")
-    hrow = np.nonzero(hc >= 0)[0]
-    hrow = hrow[np.argsort(hc[hrow], kind="stable")]
-    hit_off = np.zeros(n + 1, dtype=np.int64)
-    np.cumsum(np.bincount(hc[hrow], minlength=n), out=hit_off[1:])
+        hrow = np.nonzero(hc >= 0)[0]
+        hrow = hrow[np.argsort(hc[hrow], kind="stable")]
 
     if getattr(hits, "taxon_codes", None) is not None:
         tlut = np.fromiter((taxonomy.index[t] for t in hits.taxon_names), dtype=np.int32, count=len(hits.taxon_names))
@@ -238,3 +265,64 @@ def pack(contig_lengths, loci, hits, taxonomy):
         contig_names=names,
         contig_lengths=np.array([contig_lengths[k] for k in names], dtype=np.int64),
         hit_row=hrow, locus_row=lrow).sort_hits()
+
+
+@dataclass
+class ResidentBatch:
+    """The batch `pack` would build, with its hit columns left in a GPU parser's device columns: Engine.score_batch builds
+    them there (wfl_upload_parsed).  Carries the host-side fields the writer and the streamed runs read; contig c's hits
+    are the parser rows [hit_src[c], hit_src[c] + its hit count)."""
+    hit_off: np.ndarray        # int64 [n+1]
+    locus_off: np.ndarray      # int64 [n+1]
+    hit_src: np.ndarray        # int64 [n]  first parser row of every contig's block
+    locus_start: np.ndarray    # int32 [L]
+    locus_end: np.ndarray      # int32 [L]
+    locus_strand: np.ndarray   # int8 [L]
+    resident: object = None    # gpu_parse.ResidentParse of the hits
+    slot_node: Optional[np.ndarray] = None   # int32 [2^20] distinct-taxon slot -> node index, -1 unused
+    contig_names: list = field(default_factory=list)
+    contig_lengths: Optional[np.ndarray] = None
+    locus_row: Optional[np.ndarray] = None
+
+    n_contigs = Batch.n_contigs
+    n_hits = Batch.n_hits
+    n_loci = Batch.n_loci
+
+    @property
+    def hit_row(self):
+        """Index of each packed hit in the HitTable.  Only annotation winners read it, and with annotation systems the
+        hits stay in file order, so this is exact wherever it is read."""
+        return block_rows(self.hit_off, self.hit_src)
+
+    def slice(self, c0, c1):
+        """Contigs [c0, c1) as an independent batch with rebased offsets (the parser rows stay where they are)."""
+        h0, l0, l1 = int(self.hit_off[c0]), int(self.locus_off[c0]), int(self.locus_off[c1])
+        cut = lambda a, lo, hi: None if a is None else a[lo:hi]
+        return ResidentBatch(
+            hit_off=self.hit_off[c0:c1 + 1] - h0, locus_off=self.locus_off[c0:c1 + 1] - l0,
+            hit_src=self.hit_src[c0:c1], locus_start=self.locus_start[l0:l1], locus_end=self.locus_end[l0:l1],
+            locus_strand=self.locus_strand[l0:l1], resident=self.resident, slot_node=self.slot_node,
+            contig_names=self.contig_names[c0:c1], contig_lengths=cut(self.contig_lengths, c0, c1),
+            locus_row=cut(self.locus_row, l0, l1))
+
+
+def pack_resident(contig_lengths, loci, hits, taxonomy):
+    """`pack` for hits whose GPU parse is still live (gpu_parse.live_resident): the contig, block and locus mapping on the
+    host, the hit columns left on the device.  `taxonomy` must already be built with the hit taxa as extra names."""
+    from .gpu_parse import TAX_SLOTS, live_resident
+    res = live_resident(hits)
+    if res is None:
+        raise ValueError("pack_resident: the hits carry no live GPU parse")
+    names, locus_off, lrow, hit_off, hit_src, hc = map_contigs(contig_lengths, loci, hits)
+    if hit_src is None:   # no rows (an empty blastout): nothing to locate
+        hit_src = np.zeros(len(names), dtype=np.int64)
+    slot_node = np.full(TAX_SLOTS, -1, np.int32)
+    if len(res.taxon_slots):
+        slot_node[res.taxon_slots] = np.fromiter((taxonomy.index[t] for t in hits.taxon_names), dtype=np.int32,
+                                                 count=len(hits.taxon_names))
+    return ResidentBatch(
+        hit_off=hit_off, locus_off=locus_off, hit_src=hit_src,
+        locus_start=np.ascontiguousarray(loci.start[lrow]), locus_end=np.ascontiguousarray(loci.end[lrow]),
+        locus_strand=np.ascontiguousarray(loci.strand[lrow]), resident=res, slot_node=slot_node,
+        contig_names=names, contig_lengths=np.array([contig_lengths[k] for k in names], dtype=np.int64),
+        locus_row=lrow)

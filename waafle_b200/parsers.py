@@ -59,6 +59,8 @@ class HitTable:
         self.qseqid_codes, self.qseqid_names = qseqid_codes, qseqid_names
         # run-length view of `qseqid` (GPU parser): rows block_starts[b] .. block_starts[b+1] share block_names[b]
         self.block_starts, self.block_names = block_starts, block_names
+        # the GPU parse whose device columns hold these hits (gpu_parse.ResidentParse), or None
+        self.resident = None
 
     def __len__(self):
         return len(self.qstart)
@@ -313,7 +315,8 @@ def _read_bytes(path):
 
 def _gpu_parse_blast(path, device, genes=None):
     """The blastout parsed on the GPU (None: the CPU reader must take the file).  `genes` = (min_overlap, min_gene_length,
-    min_scov): gene calls over the parsed columns before the parser goes, returned as (HitTable, genes).  A BGZF blastout
+    min_scov): gene calls over the parsed columns, returned as (HitTable, genes).  The parser stays open with the hit
+    columns on the device (HitTable.resident): the caller closes it (close_resident) once it has scored.  A BGZF blastout
     is inflated on the device (its compressed bytes cross PCIe, not the text); other compressed files are inflated on
     the host.  A BGZF member that fails validation on the device sends the file to the CPU reader, which raises the error
     Python's gzip raises on it."""
@@ -337,11 +340,21 @@ def _gpu_parse_blast(path, device, genes=None):
         else:
             hits = parser.parse(text)
         calls = parser.call_genes(*genes) if genes is not None and hits is not None else None
-    finally:
+    except BaseException:
         parser.close()
-    if hits is not None:
+        raise
+    if hits is None:
+        parser.close()
+    else:
         hits.parse_times = parser.times
     return hits if genes is None else (hits, calls)
+
+
+def close_resident(hits):
+    """Close the GPU parser that holds the device columns of `hits`, if any."""
+    r = getattr(hits, "resident", None)
+    if r is not None:
+        r.parser.close()
 
 
 def read_blast_hits_and_genes(path, min_overlap, min_gene_length, min_scov, device=0, cpu_parse=False):

@@ -229,12 +229,13 @@ def details_order(batch, hits, contig_lengths):
     return [index[nm] for nm in dict.fromkeys(chunk_contigs(hits, contig_lengths)) if nm in index]
 
 
-def pack_chunk(names, contig_lengths, loci_index, hits, tax):
-    """packing.pack restricted to the contigs `names` (FASTA-known ones); loci rows refer to the FULL locus table."""
+def pack_chunk(names, contig_lengths, loci_index, hits, tax, pack=packing.pack):
+    """`pack` (packing.pack or packing.pack_resident) restricted to the contigs `names` (FASTA-known ones); loci rows
+    refer to the FULL locus table."""
     known = [nm for nm in dict.fromkeys(names) if nm in contig_lengths]
     sub_lengths = {nm: contig_lengths[nm] for nm in known}
     sub_loci, rows = loci_index.subset(known)
-    batch = packing.pack(sub_lengths, sub_loci, hits, tax)
+    batch = pack(sub_lengths, sub_loci, hits, tax)
     batch.locus_row = rows[batch.locus_row] if len(rows) else batch.locus_row
     return batch
 
@@ -396,12 +397,15 @@ class ChunkScorer:
             tax_changed = True
         else:
             tax_changed = False
+        # hits parsed on this worker's GPU: the batch's hit columns are built there from the parser's columns
+        from .gpu_parse import live_resident
+        pack = packing.pack_resident if live_resident(hits) is not None else packing.pack
         if loci is None:
-            batch = pack_chunk(names, self.contig_lengths, self.loci_index, hits, self.tax)
+            batch = pack_chunk(names, self.contig_lengths, self.loci_index, hits, self.tax, pack)
             loci = self.loci_index.loci
         else:
-            batch = packing.pack({nm: self.contig_lengths[nm] for nm in dict.fromkeys(names) if nm in self.contig_lengths},
-                                 loci, hits, self.tax)
+            batch = pack({nm: self.contig_lengths[nm] for nm in dict.fromkeys(names) if nm in self.contig_lengths},
+                         loci, hits, self.tax)
         n_sys = len(hits.systems)
         if self.engine is None:
             self.engine = self.Engine(self.device, self.params_factory(n_sys), self.tax)
